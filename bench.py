@@ -2,6 +2,7 @@
 """bench.py -- candidate pairs scored per second on Yelp-shaped synthetic inputs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2|C3|C4|C5] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: every pair of the workload gets the seven
 reference outputs (u_cn,u_jaccard,u_adamic,b_cn,b_jaccard,b_adamic,pa; the two union sizes are
@@ -30,6 +31,11 @@ membership ("fair", BASELINE.md section 2) on a C2 subsample; the faithful list-
 the reference's own code (oracle/_ref) on C1, the vectorised oracle and the plain-C port (one
 thread / every core, the latter over ALL pairs and compared with the GPU's output) sit beside it.
 `--impl reference` prints the all-core CPU arm as its own line.
+
+`--dump-outputs DIR` writes what the last timed step computed -- every column the timed call
+returns (N>1: rank 0's window) -- as DIR/<column>.npy in float64, which holds the integer columns
+exactly.  Above DUMP_ROWS rows it writes a fixed seeded sample of rows, the same for every run with
+the same arguments; DIR/row_index.npy says which.  Two builds can so be compared output for output.
 """
 import argparse
 import importlib
@@ -46,6 +52,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree, which may be read-only
 PKG = 'bipartite-link-prediction_b200'
 METRIC = 'candidate pairs scored/sec'
 UNIT = 'pairs/s'
@@ -277,6 +284,27 @@ def compare_with_oracle(host, want):
             'ok': not bad}
 
 
+# --dump-outputs: at most 2^19 rows of each of at most ten arrays, 8 B each: 42 MB in all
+DUMP_ROWS = 1 << 19
+
+
+def dump_rows(n):
+    """The rows --dump-outputs writes: all n, or a fixed seeded sample of DUMP_ROWS, ascending."""
+    if n <= DUMP_ROWS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(n, size=DUMP_ROWS, replace=False))
+
+
+def dump_outputs(path, cols, rows):
+    """cols: column name -> device tensor of every row; writes rows `rows` of each as float64."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    t_rows = torch.from_numpy(rows).to(next(iter(cols.values())).device)
+    np.save(os.path.join(path, 'row_index.npy'), rows.astype(np.float64))
+    for k, v in cols.items():
+        np.save(os.path.join(path, k + '.npy'), v[t_rows].cpu().numpy().astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------ clocks
 class ClockSampler(object):
     Q = ('clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,'
@@ -477,7 +505,14 @@ def main():
     ap.add_argument('--derive', default=None, help="N>1: comma list of columns rank 0 derives (default pa)")
     ap.add_argument('--quick', action='store_true',
                     help='headline measurement and checks only: no comparison arms, no e2e, no other configs')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step to DIR/<column>.npy (float64; a '
+                         'fixed seeded sample of %d rows when there are more)' % DUMP_ROWS)
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'b200':
+        ap.error('--dump-outputs writes what the GPU path computed; it does not apply to --impl %s' % a.impl)
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -523,7 +558,7 @@ def main():
             return
         t0 = time.perf_counter()
         vals = []
-        for _ in range(max(1, min(a.steps, 2))):
+        for _ in range(a.steps):
             rate, sample, sides = cpu_reference_all_cores(cfg, eu, eb, pu, pv, ug, bg, cores)
             vals.append(rate)
         rate = statistics.median(vals)
@@ -673,6 +708,10 @@ def main():
     barrier()                              # N>1: every rank's rows are on rank 0 from here on
     t_wall1 = time.perf_counter()
     clocks = sampler.window(t_wall0, t_wall1) if sampler else None
+    if a.dump_outputs and rank == 0:
+        # now: the comparison arms below reuse these buffers
+        dump_outputs(a.dump_outputs, window.tensors() if window is not None else outs,
+                     dump_rows(n_total))
     ms_per_step = reduce_max(total_ms) / a.steps
     value = n_total / (ms_per_step * 1e-3)
     wall_ms_per_step = reduce_max((t_wall1 - t_wall0) * 1e3) / a.steps

@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -19,17 +21,33 @@ def test_library_exports_every_declared_symbol(built_lib):
     assert built_lib.blp_version() >= 100
 
 
+NO_DEVICE_CHECKS = r'''
+import ctypes
+import sys
+import torch
+sys.path.insert(0, sys.argv[1])
+from conftest import pkg
+assert not torch.cuda.is_available()
+lib_mod = pkg('_lib')
+lib = lib_mod.load()
+n = ctypes.c_int(-1)
+assert lib.blp_device_count(ctypes.byref(n)) == lib_mod.BLP_ERR_CUDA and n.value == 0
+assert b'CUDA' in lib.blp_last_error()
+try:
+    pkg('graph').BipartiteGraph(4, 3, [0, 1], [0, 1])       # fails loudly, never computes on CPU
+except RuntimeError:
+    pass
+else:
+    raise AssertionError('BipartiteGraph was created without a CUDA device')
+'''
+
+
 def test_no_cpu_fallback_without_device(built_lib):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip('a CUDA device is present')
-    lib_mod = pkg('_lib')
-    n = ctypes.c_int(-1)
-    assert built_lib.blp_device_count(ctypes.byref(n)) == lib_mod.BLP_ERR_CUDA and n.value == 0
-    assert b'CUDA' in built_lib.blp_last_error()
-    graph = pkg('graph')
-    with pytest.raises(RuntimeError):                       # fails loudly, never computes on CPU
-        graph.BipartiteGraph(4, 3, [0, 1], [0, 1])
+    """Run in a child process that sees no CUDA device, so that it runs on GPU machines too."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES='')
+    res = subprocess.run([sys.executable, '-c', NO_DEVICE_CHECKS, os.path.join(ROOT, 'tests')], env=env,
+                         stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
+    assert res.returncode == 0, res.stdout[-4000:]
 
 
 def test_argument_validation_precedes_device_use(built_lib):
