@@ -20,6 +20,7 @@ SOURCES = ('blp_graph.cu', 'blp_build.cu', 'blp_score.cu', 'blp_host.cu', 'blp_h
 BLP_OK = 0
 BLP_ERR_INVALID, BLP_ERR_CUDA, BLP_ERR_OOM, BLP_ERR_RANGE, BLP_ERR_UNSUPPORTED = -1, -2, -3, -4, -5
 SIDE_USER, SIDE_BUSINESS = 0, 1
+PATH_GROUPED, PATH_BIZ_INDEX = 0, 1     # blp_score_stats_t.path
 
 # every symbol include/blp.h declares
 EXPORTS = ('blp_version', 'blp_last_error', 'blp_device_count', 'blp_graph_create',
@@ -40,7 +41,8 @@ class GraphInfo(ctypes.Structure):
                 ('device_bytes', ctypes.c_int64), ('device', ctypes.c_int32),
                 ('sm_count', ctypes.c_int32), ('n_hub_biz', ctypes.c_int32),
                 ('n_hub_users', ctypes.c_int32), ('hub_min_biz_degree', ctypes.c_int32),
-                ('hub_min_user_degree', ctypes.c_int32)]
+                ('hub_min_user_degree', ctypes.c_int32), ('biz_index_bytes', ctypes.c_int64),
+                ('biz_index_build_ms', ctypes.c_float)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -52,7 +54,7 @@ class ScoreStats(ctypes.Structure):
                 ('threads_per_cta', ctypes.c_int32), ('smem_bytes', ctypes.c_int32),
                 ('range_passes', ctypes.c_int32), ('group_ms', ctypes.c_float),
                 ('score_ms', ctypes.c_float), ('light_ms', ctypes.c_float),
-                ('light_groups', ctypes.c_int32)]
+                ('light_groups', ctypes.c_int32), ('path', ctypes.c_int32)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}

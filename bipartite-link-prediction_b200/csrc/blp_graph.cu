@@ -225,6 +225,8 @@ void read_tuning(blp_tuning* t) {
     if (const char* e = getenv("BLP_SLICE_GROWTH")) t->slice_growth = atof(e);
     if (getenv("BLP_NO_BANK_STRIPE")) t->bank_stripe = false;
     if (const char* e = getenv("BLP_HOP3_GLOBAL")) t->hop3_global = atoi(e) != 0;
+    if (const char* e = getenv("BLP_BIZ_INDEX")) t->biz_index = atoi(e) != 0 ? 1 : 0;
+    if (const char* e = getenv("BLP_BIZ_INDEX_MAX_MB")) t->biz_index_cap = atoll(e) << 20;
 }
 
 // 1/ln(d) in Q1.31 for d = 0..max_deg (0 for d <= 1), evaluated with the host libm.
@@ -428,6 +430,9 @@ extern "C" int blp_graph_destroy(blp_graph* g) {
         cudaFree(g->hubtab_cn[sd]);
         cudaFree(g->hubtab_aa[sd]);
     }
+    cudaFree(g->biz_index);
+    cudaFree(g->biz_hop2);
+    cudaFree(g->biz_radj);
     for (int sd = 0; sd < 2; ++sd)
         for (int k = 0; k < 4; ++k)
             if (g->ev[sd][k]) cudaEventDestroy(g->ev[sd][k]);
@@ -461,6 +466,8 @@ extern "C" int blp_graph_info(const blp_graph* g, blp_graph_info_t* info) {
     info->n_hub_users = g->n_hubs[1];
     info->hub_min_biz_degree = g->n_hubs[0] ? g->hub_min_deg[0] : 0;
     info->hub_min_user_degree = g->n_hubs[1] ? g->hub_min_deg[1] : 0;
+    info->biz_index_bytes = g->biz_index ? g->biz_index_bytes : 0;
+    info->biz_index_build_ms = g->biz_index ? g->biz_index_build_ms : 0.f;
     return BLP_OK;
 }
 
@@ -491,7 +498,12 @@ extern "C" int blp_score_stats(const blp_graph* g, int side, blp_score_stats_t* 
         return BLP_ERR_INVALID;
     }
     *stats = g->stats[side];
-    if (g->ev_recorded[side]) {
+    if (g->ev_recorded[side] && stats->path == BLP_PATH_BIZ_INDEX) {
+        // one kernel, no grouping: its time is the whole call's
+        BLP_ON_DEVICE(g->device);
+        BLP_CUDA_TRY(cudaEventSynchronize(g->ev[side][2]));
+        BLP_CUDA_TRY(cudaEventElapsedTime(&stats->score_ms, g->ev[side][1], g->ev[side][2]));
+    } else if (g->ev_recorded[side]) {
         BLP_ON_DEVICE(g->device);
         BLP_CUDA_TRY(cudaEventSynchronize(g->ev[side][2]));
         BLP_CUDA_TRY(cudaEventElapsedTime(&stats->group_ms, g->ev[side][0], g->ev[side][1]));

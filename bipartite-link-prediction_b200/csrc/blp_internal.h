@@ -32,6 +32,8 @@ struct blp_tuning {
     double slice_growth = 0.0; // BLP_SLICE_GROWTH: user-side slice plan of blp_score_pairs_host
     bool bank_stripe = true;   // BLP_NO_BANK_STRIPE: leave long rows in ascending order
     bool hop3_global = false;  // BLP_HOP3_GLOBAL=1: hop-3 user bitmap in global scratch even when it fits shared memory
+    int biz_index = -1;        // BLP_BIZ_INDEX=0|1: never / always (cap ignored) build the business index (-1 = by size)
+    long long biz_index_cap = 0;  // BLP_BIZ_INDEX_MAX_MB: byte cap of the automatic choice (0 = default)
 };
 
 struct blp_graph {
@@ -99,6 +101,19 @@ struct blp_graph {
     int n_hubs[2] = {0, 0};                           // bitmaps kept (both kinds)
     int probe_ratio = 2;                              // probe when deg(y) >= ratio * |hop2(x)|
     bool row_slots[2] = {false, false};               // slot bits present in the middle rows of side s
+    // Business index: the business x business co-review relation as one bitmap row per business,
+    // row b = hop2(b) (businesses sharing a reviewer with b, b itself excluded), biz_index_words
+    // words each, and |hop2(b)| per business.  Built once per graph when the business side runs
+    // unranged and the rows fit the cap (build_biz_index); the business side then scores every
+    // pair by testing N(u) against row b, with no grouping.  nullptr = the grouped path.
+    // Its columns are business RANKS by degree (blp_score_index.cuh); biz_radj = u_adj with every
+    // business id replaced by its rank.
+    unsigned* biz_index = nullptr;
+    int* biz_hop2 = nullptr;
+    int* biz_radj = nullptr;
+    int biz_index_words = 0;
+    int64_t biz_index_bytes = 0;
+    float biz_index_build_ms = 0.f;
     blp_score_stats_t stats[2] = {};
     cudaEvent_t ev[2][4] = {};   // per side: start, after grouping, after scoring, after the light kernel
     bool ev_light[2] = {false, false};

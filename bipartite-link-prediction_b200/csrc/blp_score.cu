@@ -12,19 +12,26 @@
 //   cn(x,y) = | { i in N(y) : i in hop2(x) } |     N(y) streamed with 128-bit loads -- or, when y
 //                                                 has a bitmap of its own, hop2(x) probed into it
 //
-// Work distribution.  Pairs are grouped by x (runs of an already grouped list, or a counting sort:
-// k_group_*), the groups are split by size class, and two persistent grids pull their groups from
-// atomic counters.  Inside a CTA of k_score_side both the expansion and the intersection
-// phase walk a *set of adjacency lists* whose lengths span 1 .. >100k: the lists of a tile are
-// cut into 512-id chunks, the chunk counts are prefix-summed in shared memory and warps take
-// chunks round-robin, so a hub list is spread over the whole CTA while short lists cost one
-// warp pass each (degree-bucketed scheduling without separate launches).
+// Work distribution.  The user side, and the business side of a handle without a business index,
+// take the GROUPED path: pairs are grouped by x (runs of an already grouped list, or a counting
+// sort: k_group_*), the groups are split by size class, and two persistent grids pull their
+// groups from atomic counters.  Inside a CTA of k_score_side both the expansion and the
+// intersection phase walk a *set of adjacency lists* whose lengths span 1 .. >100k: the lists of
+// a tile are cut into 512-id chunks, the chunk counts are prefix-summed in shared memory and warps
+// take chunks round-robin, so a hub list is spread over the whole CTA while short lists cost one
+// warp pass each (degree-bucketed scheduling without separate launches).  The business side of a
+// handle WITH an index (hop2(b) of every business precomputed once per graph as a bitmap row:
+// C1-C4) is one pass over the pairs in the caller's order, k_score_biz_indexed: a lane tests N(u)
+// against row b, the warp walks the rare long N(u) together -- no grouping, no expansion, no
+// un-permute.  Both paths end in the same epilogue (emit_pair).
 //
 // Layout of the translation unit:
-//   blp_score_common.cuh  launch arguments (SideArgs), row-descriptor accessors, streaming loads
+//   blp_score_common.cuh  launch arguments (SideArgs), row-descriptor accessors, streaming loads,
+//                         the shared epilogue
 //   blp_score_group.cuh   pairs -> work items (runs / counting sort), light / heavy split
 //   blp_score_light.cuh   k_score_light: one WARP per small group (hash-table hop-2 set), the
 //                         per-node class flags and the hub x bitmap-node intersection tables
+//   blp_score_index.cuh   the business index: its construction and the per-pair kernel
 //   this file             k_score_side: one CTA per group (shared-memory bitmap), hub-bitmap
 //                         construction, blp_score_pairs (grouping, split, both launches)
 #include <algorithm>
@@ -44,6 +51,7 @@
 #include "blp_score_common.cuh"
 #include "blp_score_group.cuh"
 #include "blp_score_light.cuh"
+#include "blp_score_index.cuh"
 
 namespace blp {
 
@@ -487,18 +495,7 @@ __global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREA
             // pairs with an id that is not in the graph: every score is the literal 0
             for (long long k = p0 + tid; k < p1; k += NT) {
                 int idx = a.pg ? a.pg[k].x : (int)k;
-                if (REC) {
-                    st_stream(a.rec + 3 * k, 0ull);
-                    st_stream(a.rec + 3 * k + 1, 0ull);
-                    st_stream(a.rec + 3 * k + 2, 0ull);
-                } else {
-                    if (a.cn) st_stream(a.cn + idx, 0);
-                    if (a.uni) st_stream(a.uni + idx, 0);
-                    if (a.jac) st_stream(a.jac + idx, 0.0);
-                    if (a.aa) st_stream(a.aa + idx, 0.0);
-                }
-                if (a.pa) st_stream(a.pa + idx, 0ll);
-                if (a.hop2) st_stream(a.hop2 + idx, 0);
+                emit_pair<REC>(a, k, idx, false, 0, 0, 0, 0, 0ull);
             }
             __syncthreads();                       // everyone is past reading ts.item_next
             if (tid == 0) ts.item_next = claimed;
@@ -717,26 +714,8 @@ __global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREA
                 }
             }
             if (tid < count && final_pass) {
-                int idx = ts.idx[tid];
-                int c = ts.cn[tid];
-                int pdeg = RANGED ? ts.hub[tid] : row_deg(ts.row[tid]);
-                int u = hop2 + pdeg - c;   // |a| + |b| - |a & b|  (similarity.py:110)
-                const double jv = __ddiv_rn((double)c, (double)u);
-                const double av = (double)ts.aa[tid] * (1.0 / (double)(1ull << BLP_AA_FRAC_BITS));
-                // results stream out once (on the multi-GPU path into a peer's memory): evict-first
-                if (REC) {
-                    unsigned long long* r = a.rec + 3 * (tb + tid);
-                    st_stream(r, (unsigned long long)(unsigned)c | ((unsigned long long)(unsigned)u << 32));
-                    st_stream(r + 1, (unsigned long long)__double_as_longlong(jv));
-                    st_stream(r + 2, (unsigned long long)__double_as_longlong(av));
-                } else {
-                    if (a.cn) st_stream(a.cn + idx, c);
-                    if (a.uni) st_stream(a.uni + idx, u);
-                    if (a.jac) st_stream(a.jac + idx, jv);
-                    if (a.aa) st_stream(a.aa + idx, av);
-                }
-                if (a.pa) st_stream(a.pa + idx, (long long)xdeg * (long long)pdeg);
-                if (a.hop2) st_stream(a.hop2 + idx, hop2);
+                const int pdeg = RANGED ? ts.hub[tid] : row_deg(ts.row[tid]);
+                emit_pair<REC>(a, tb + tid, ts.idx[tid], true, ts.cn[tid], hop2, xdeg, pdeg, ts.aa[tid]);
             }
             __syncthreads();
             BLP_TICK(8);
@@ -832,6 +811,7 @@ __global__ void k_build_hub_bitmaps(const int* __restrict__ hub_nodes, int n_hub
 // final list walker (batched probes, counted atomics) the optimum sits at bm_bytes/30
 // (user side: deg >= 1016 6.71 ms, >= 1500 6.50 ms, >= 2500 6.56 ms; business side flat).
 int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host) {
+    reserve_biz_index(g);   // first: with an index the business side needs no tables or flags
     for (int side = 0; side < 2; ++side) {
         const bool us = side == BLP_SIDE_USER;
         const int n_side = us ? g->n_users : g->n_biz;     // bitmap universe
@@ -928,7 +908,8 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
         // skipped when they would take more than ~2e9 probes to fill
         long long or_ids = 0;
         for (int m : or_nodes) or_ids += mdeg[m];
-        if (probing && !or_nodes.empty() && or_ids * (long long)hubs.size() <= 2000000000LL) {
+        const bool grouped = us || !g->biz_index;   // the tables serve the grouped path only
+        if (grouped && probing && !or_nodes.empty() && or_ids * (long long)hubs.size() <= 2000000000LL) {
             const size_t cells = or_nodes.size() * hubs.size();
             int* d_or = nullptr;
             BLP_CUDA_TRY(cudaMalloc((void**)&d_or, sizeof(int) * or_nodes.size()));
@@ -951,7 +932,7 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
         for (int side = 0; side < 2; ++side) {
             const bool us = side == BLP_SIDE_USER;
             const int n_side = us ? g->n_users : g->n_biz;
-            if (n_side <= 0) continue;
+            if (n_side <= 0 || (!us && g->biz_index)) continue;
             const unsigned long long* g_row = (const unsigned long long*)(us ? g->u_row : g->b_row);
             const unsigned long long* m_row = (const unsigned long long*)(us ? g->b_row : g->u_row);
             BLP_CUDA_TRY(cudaMalloc((void**)&g->light[side], (size_t)n_side));
@@ -966,7 +947,7 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
         }
         BLP_CUDA_TRY(cudaDeviceSynchronize());
     }
-    return BLP_OK;
+    return build_biz_index(g, b_deg_host);
 }
 
 }  // namespace blp
@@ -1019,6 +1000,7 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
     a.aa = adamic;
     a.pa = (long long*)pa;
     a.hop2 = hop2_size;
+    if (!us && g->biz_index) return score_biz_indexed(g, a, pair_u, pair_b, n, st);
 
     // id-range passes: planned when the handle was created (range_plan), because the middle rows
     // of a ranged side are laid out partitioned by range

@@ -232,6 +232,42 @@ __device__ __forceinline__ unsigned long long segment_row(const SideArgs& a, uns
     return ((unsigned long long)f4 << 24) | (unsigned)(n4 << 2);
 }
 
+// The epilogue every scoring kernel shares: one pair's integer counts -> its result columns.
+// c = |hop2(x) & N(y)|, aa_q = the Q1.31 weight sum over those ids, pdeg = deg(y), xdeg = deg(x).
+// valid = false is the "id not in graph" bucket (similarity.py:52,59-60): every output, hop2
+// included, is the literal 0.  REC: the record at grouped position k instead of the caller-order
+// columns (pa and hop2 always go to the caller-order index idx).
+template <bool REC>
+__device__ __forceinline__ void emit_pair(const SideArgs& a, long long k, int idx, bool valid, int c,
+                                          int hop2, int xdeg, int pdeg, unsigned long long aa_q) {
+    int u = 0;
+    double jv = 0.0, av = 0.0;
+    long long pa = 0;
+    if (valid) {
+        u = hop2 + pdeg - c;   // |a| + |b| - |a & b|  (similarity.py:110)
+        jv = __ddiv_rn((double)c, (double)u);
+        av = (double)aa_q * (1.0 / (double)(1ull << BLP_AA_FRAC_BITS));
+        pa = (long long)xdeg * (long long)pdeg;
+    } else {
+        c = 0;
+        hop2 = 0;
+    }
+    // results stream out once (on the multi-GPU path into a peer's memory): evict-first
+    if (REC) {
+        unsigned long long* r = a.rec + 3 * k;
+        st_stream(r, (unsigned long long)(unsigned)c | ((unsigned long long)(unsigned)u << 32));
+        st_stream(r + 1, (unsigned long long)__double_as_longlong(jv));
+        st_stream(r + 2, (unsigned long long)__double_as_longlong(av));
+    } else {
+        if (a.cn) st_stream(a.cn + idx, c);
+        if (a.uni) st_stream(a.uni + idx, u);
+        if (a.jac) st_stream(a.jac + idx, jv);
+        if (a.aa) st_stream(a.aa + idx, av);
+    }
+    if (a.pa) st_stream(a.pa + idx, pa);
+    if (a.hop2) st_stream(a.hop2 + idx, hop2);
+}
+
 constexpr int kShortV4 = 4;   // lists of <= 16 ids take the sub-warp path (4 lanes per list)
 // Probe path.  A hop-2 set built from at most kProbeCap list entries and no hub bitmap is also
 // kept as an id list (the atomicOr that turns a bit on appends the id).  A pair of that group

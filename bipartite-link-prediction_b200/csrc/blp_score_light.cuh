@@ -409,26 +409,8 @@ __global__ void __launch_bounds__(WARPS * 32, BLP_LIGHT_MIN_CTAS) k_score_light(
                 }
             }
             if (tb == p0) light_stage_d(a, nxt, lane);
-            // epilogue: same expressions as k_score_side
-            if (lane < count) {
-                const int cnn = (int)my_cn;
-                const int u = hop2 + pdeg - cnn;   // |a| + |b| - |a & b|  (similarity.py:110)
-                const double jv = __ddiv_rn((double)cnn, (double)u);
-                const double av = (double)my_aa * (1.0 / (double)(1ull << BLP_AA_FRAC_BITS));
-                if (REC) {
-                    unsigned long long* rr = a.rec + 3 * (tb + lane);
-                    st_stream(rr, (unsigned long long)(unsigned)cnn | ((unsigned long long)(unsigned)u << 32));
-                    st_stream(rr + 1, (unsigned long long)__double_as_longlong(jv));
-                    st_stream(rr + 2, (unsigned long long)__double_as_longlong(av));
-                } else {
-                    if (a.cn) st_stream(a.cn + idx, cnn);
-                    if (a.uni) st_stream(a.uni + idx, u);
-                    if (a.jac) st_stream(a.jac + idx, jv);
-                    if (a.aa) st_stream(a.aa + idx, av);
-                }
-                if (a.pa) st_stream(a.pa + idx, (long long)xdeg * (long long)pdeg);
-                if (a.hop2) st_stream(a.hop2 + idx, hop2);
-            }
+            // epilogue: the one every scoring kernel uses
+            if (lane < count) emit_pair<REC>(a, tb + lane, idx, true, (int)my_cn, hop2, xdeg, pdeg, my_aa);
             __syncwarp();
         }
         if (p0 >= p1) {   // (never: an item has at least one pair)

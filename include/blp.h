@@ -68,7 +68,16 @@ typedef struct blp_graph_info_t {
     int32_t n_hub_users;      /* users whose business list is also kept as a bitmap (business side) */
     int32_t hub_min_biz_degree;
     int32_t hub_min_user_degree;
+    int64_t biz_index_bytes;     /* business x business co-review bitmap (0 = not built: the
+                                    business side groups and expands per call) */
+    float biz_index_build_ms;    /* its construction time at graph creation */
 } blp_graph_info_t;
+
+/* Which kernels scored the last call of a side (blp_score_stats_t.path). */
+typedef enum blp_score_path {
+    BLP_PATH_GROUPED = 0,   /* pairs grouped by x, hop2(x) built per group (k_score_side / k_score_light) */
+    BLP_PATH_BIZ_INDEX = 1  /* business side: one pass over the pairs against the co-review bitmap */
+} blp_score_path;
 
 /* Per-launch accounting of the last blp_score_pairs call on a handle (for bench / roofline). */
 typedef struct blp_score_stats_t {
@@ -83,6 +92,7 @@ typedef struct blp_score_stats_t {
     float score_ms;           /* CUDA-event time of the scoring kernels alone, on their own stream */
     float light_ms;           /* span of the warp-per-group kernel (it runs beside the CTA kernel), 0 if not used */
     int32_t light_groups;     /* work items scored by the warp-per-group kernel */
+    int32_t path;             /* blp_score_path */
 } blp_score_stats_t;
 
 int blp_version(void);
