@@ -12,8 +12,6 @@ _ROOT = os.path.dirname(_HERE)
 CSRC = os.path.join(_HERE, 'csrc')
 INCLUDE = os.path.join(_ROOT, 'include')
 LIB_PATH = os.path.join(_HERE, 'libblp.so')
-if os.environ.get('BLP_LIB_PATH'):        # developer override: A/B a prebuilt variant (tools/build_variants.py)
-    LIB_PATH = os.path.abspath(os.environ['BLP_LIB_PATH'])
 SOURCES = ('blp_graph.cu', 'blp_build.cu', 'blp_score.cu', 'blp_host.cu', 'blp_hop3.cu', 'blp_eval.cu',
            'blp_peer.cu')
 

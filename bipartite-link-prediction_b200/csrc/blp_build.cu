@@ -746,7 +746,7 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
         if (rc__ != BLP_OK) return fail(rc__); \
     } while (0)
 
-    BLP_RC_B(init_device_state(g, device));
+    BLP_RC_B(init_device_state(g, device, read_tuning()));
 
     // ---- keys, validity
     unsigned long long *keys = nullptr, *keys2 = nullptr, *pos = nullptr, *edges = nullptr;
@@ -862,12 +862,10 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
                                                            (unsigned long long*)g->b_row, g->b_deg);
     // a side that needs id-range passes gets its middle rows partitioned by range instead of
     // bank-striped: business rows serve the user side, user rows the business side
-    if (g->tune.bank_stripe) {   // (BLP_NO_BANK_STRIPE, read at handle creation)
-        if (g->n_ranges[1] == 1)
-            k_bank_stripe<<<g->sm_count * 4, 256, 0, st>>>(u_off, u_deg, n_users, g->u_adj, tmp, next_row);
-        if (g->n_ranges[0] == 1)
-            k_bank_stripe<<<g->sm_count * 4, 256, 0, st>>>(b_off, b_deg, n_biz, g->b_adj, tmp, next_row + 1);
-    }
+    if (g->n_ranges[1] == 1)
+        k_bank_stripe<<<g->sm_count * 4, 256, 0, st>>>(u_off, u_deg, n_users, g->u_adj, tmp, next_row);
+    if (g->n_ranges[0] == 1)
+        k_bank_stripe<<<g->sm_count * 4, 256, 0, st>>>(b_off, b_deg, n_biz, g->b_adj, tmp, next_row + 1);
     BLP_TRY_B(cudaGetLastError());
     BLP_RC_B(build_range_segments(g, /*reorder=*/true, tmp, st));
 

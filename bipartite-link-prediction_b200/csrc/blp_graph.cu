@@ -192,14 +192,15 @@ void release_scratch_pool(int device) {
     }
 }
 
-// Device properties, the scratch pool and the timing events of a new handle.
-int init_device_state(blp_graph* g, int device) {
+// Device properties, tuning (read_tuning, called once by the builder), the scratch pool and the
+// timing events of a new handle.
+int init_device_state(blp_graph* g, int device, const blp_tuning& tune) {
     cudaDeviceProp prop;
     BLP_CUDA_TRY(cudaGetDeviceProperties(&prop, device));
     g->device = device;
     g->sm_count = prop.multiProcessorCount;
     g->max_smem_optin = (int)prop.sharedMemPerBlockOptin;
-    read_tuning(&g->tune);
+    g->tune = tune;
     g->pool = acquire_scratch_pool(device);   // nullptr: fall back to the default pool, untouched
     for (int sd = 0; sd < 2; ++sd)
         for (int k = 0; k < 4; ++k) BLP_CUDA_TRY(cudaEventCreate(&g->ev[sd][k]));
@@ -216,17 +217,18 @@ int init_device_state(blp_graph* g, int device) {
     return BLP_OK;
 }
 
-void read_tuning(blp_tuning* t) {
-    if (const char* e = getenv("BLP_RANGES")) t->ranges = atoi(e);
-    if (const char* e = getenv("BLP_GROUPING"))
-        t->grouping = !strcmp(e, "runs") ? 1 : (!strcmp(e, "sort") ? 0 : -1);   // MODE_RUNS / MODE_SORT
-    if (const char* e = getenv("BLP_NT")) t->nt = atoi(e);
-    if (const char* e = getenv("BLP_LIGHT_STREAM")) t->light_stream = atoi(e) != 0;
-    if (const char* e = getenv("BLP_SLICE_GROWTH")) t->slice_growth = atof(e);
-    if (getenv("BLP_NO_BANK_STRIPE")) t->bank_stripe = false;
-    if (const char* e = getenv("BLP_HOP3_GLOBAL")) t->hop3_global = atoi(e) != 0;
-    if (const char* e = getenv("BLP_BIZ_INDEX")) t->biz_index = atoi(e) != 0 ? 1 : 0;
-    if (const char* e = getenv("BLP_BIZ_INDEX_MAX_MB")) t->biz_index_cap = atoll(e) << 20;
+blp_tuning read_tuning() {
+    blp_tuning t;
+    if (const char* e = getenv("BLP_RANGES")) t.ranges = atoi(e);
+    if (const char* e = getenv("BLP_HUB_MIN_DEG")) t.hub_min_deg = std::max(0, atoi(e));
+    if (const char* e = getenv("BLP_PROBE_MIN_DEG")) t.probe_min_deg = std::max(0, atoi(e));
+    if (const char* e = getenv("BLP_PROBE_RATIO")) t.probe_ratio = std::max(1, atoi(e));
+    if (const char* e = getenv("BLP_LIGHT")) t.light = atoi(e) != 0;
+    if (const char* e = getenv("BLP_LIGHT_HUBS")) t.light_hubs = atoi(e) != 0;
+    if (const char* e = getenv("BLP_HOP3_GLOBAL")) t.hop3_global = atoi(e) != 0;
+    if (const char* e = getenv("BLP_BIZ_INDEX")) t.biz_index = atoi(e) != 0 ? 1 : 0;
+    if (const char* e = getenv("BLP_BIZ_INDEX_MAX_MB")) t.biz_index_cap = atoll(e) << 20;
+    return t;
 }
 
 // 1/ln(d) in Q1.31 for d = 0..max_deg (0 for d <= 1), evaluated with the host libm.
@@ -329,15 +331,14 @@ extern "C" int blp_graph_create(int32_t n_users, int32_t n_biz, int64_t n_edges,
             }
         }
         std::vector<uint64_t>().swap(keys);
-        blp_tuning tune;
-        blp::read_tuning(&tune);
+        const blp_tuning tune = blp::read_tuning();
         // a side that needs id-range passes keeps its middle rows ascending (= partitioned by
         // range): business rows serve the user side, user rows the business side
         int optin = 0, nr_user = 1, nr_biz = 1, rw = 0;
         BLP_CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
         blp::range_plan(n_users, optin, tune.ranges, &nr_user, &rw);
         blp::range_plan(n_biz, optin, tune.ranges, &nr_biz, &rw);
-        if (tune.bank_stripe) {   // (BLP_NO_BANK_STRIPE: tuning switch)
+        {
             std::vector<int32_t> tmp;
             std::vector<int32_t> bucket[32];
             if (nr_biz == 1)
@@ -382,7 +383,7 @@ extern "C" int blp_graph_create(int32_t n_users, int32_t n_biz, int64_t n_edges,
         blp::entry_weights(u_adj, n_biz, b_deg, g->max_bdeg, u_adjw);   // user rows name businesses
         blp::entry_weights(b_adj, n_users, u_deg, g->max_udeg, b_adjw); // business rows name users
 
-        rc = blp::init_device_state(g, device);
+        rc = blp::init_device_state(g, device, tune);
         if (rc == BLP_OK) rc = blp::upload(&g->u_row, u_row, &g->device_bytes);
         if (rc == BLP_OK) rc = blp::upload(&g->b_row, b_row, &g->device_bytes);
         if (rc == BLP_OK) rc = blp::upload(&g->u_adj, u_adj, &g->device_bytes);

@@ -11,7 +11,6 @@
 // the next slice's scoring.  Native on purpose: issuing ~100 launches and ~100 copies per step
 // from Python costs more than a millisecond of host time during which the GPU starves.
 #include <algorithm>
-#include <cmath>
 #include <cstdlib>
 #include <vector>
 
@@ -109,14 +108,11 @@ extern "C" int blp_score_pairs_host(blp_graph* g, const int32_t* pair_u, const i
     const int uc = std::max(1, std::min(user_slices > 0 ? user_slices : 4, max_slices));
     const int bc = std::max(1, std::min(biz_slices > 0 ? biz_slices : 2, max_slices));
     const int lead = std::max(0, std::min(lead_slices >= 0 ? lead_slices : 1, uc - 1));
-    const double slice_growth = g->tune.slice_growth;   // (BLP_SLICE_GROWTH, read at handle creation)
-    // equal user-side slices by default; BLP_SLICE_GROWTH = g > 1 puts bound c at n * (c/uc)^g
-    // (small first slice, larger later ones) -- measured slower on C2 for g = 1.5 and 2
-    const double grow = slice_growth > 0 ? slice_growth : 1.0;
+    // equal user-side slices, bounds on multiples of four pairs (growing slices, a small first one
+    // and larger later ones, measured slower on C2)
     auto ubound = [&](int c) {
         if (c >= uc) return n;
-        const double f = pow((double)c / (double)uc, grow);
-        return std::min<int64_t>(n, (int64_t)((double)n * f) / 4 * 4);
+        return std::min<int64_t>(n, (int64_t)((double)n * ((double)c / uc)) / 4 * 4);
     };
     auto bbound = [&](int c) { return n * c / bc; };
 

@@ -26,11 +26,11 @@ struct blp_host_state;   // staging buffers and streams of blp_score_pairs_host 
 // the scoring path.
 struct blp_tuning {
     int ranges = 0;            // BLP_RANGES: at least this many id-range passes
-    int grouping = -1;         // BLP_GROUPING=runs|sort: force a grouping mode (-1 = decide on the device)
-    int nt = 0;                // BLP_NT=256|512|1024: threads per CTA of k_score_side (0 = by size)
-    bool light_stream = true;  // BLP_LIGHT_STREAM=0: keep k_score_light on the caller's stream
-    double slice_growth = 0.0; // BLP_SLICE_GROWTH: user-side slice plan of blp_score_pairs_host
-    bool bank_stripe = true;   // BLP_NO_BANK_STRIPE: leave long rows in ascending order
+    int hub_min_deg = -1;      // BLP_HUB_MIN_DEG: hub bitmaps from this degree on (0 = none, -1 = by bitmap size)
+    int probe_min_deg = -1;    // BLP_PROBE_MIN_DEG: probe bitmaps from this degree on (0 = none, -1 = by hub degree)
+    int probe_ratio = 0;       // BLP_PROBE_RATIO: probe when deg(y) >= ratio * |hop2(x)| (0 = kProbeRatio)
+    bool light = true;         // BLP_LIGHT=0: no warp-per-group kernel
+    bool light_hubs = true;    // BLP_LIGHT_HUBS=0: the warp-per-group kernel takes hub-free groups only
     bool hop3_global = false;  // BLP_HOP3_GLOBAL=1: hop-3 user bitmap in global scratch even when it fits shared memory
     int biz_index = -1;        // BLP_BIZ_INDEX=0|1: never / always (cap ignored) build the business index (-1 = by size)
     long long biz_index_cap = 0;  // BLP_BIZ_INDEX_MAX_MB: byte cap of the automatic choice (0 = default)
@@ -133,14 +133,14 @@ constexpr int kMaxRanges = 255;
 // partition the middle rows of every ranged side by id range (reorder = false: rows already ascend)
 // and fill seg_off; `tmp` = scratch of max(u_adj_len, b_adj_len) ints when reordering
 int build_range_segments(blp_graph* g, bool reorder, int* tmp, cudaStream_t st);
-int init_device_state(blp_graph* g, int device);
+int init_device_state(blp_graph* g, int device, const blp_tuning& tune);
 void host_state_destroy(blp_graph* g);
 void weight_lut(int32_t max_deg, std::vector<unsigned>& lut);
 int radix_sort_u64(unsigned long long* keys, unsigned long long* tmp, long long n,
                    const std::vector<int>& shifts, cudaStream_t st, unsigned long long** sorted);
 void set_error(const std::string& msg);
 int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
-void read_tuning(blp_tuning* t);
+blp_tuning read_tuning();
 cudaMemPool_t acquire_scratch_pool(int device);
 void release_scratch_pool(int device);
 cudaError_t scratch_alloc(void** p, size_t bytes, cudaStream_t st);

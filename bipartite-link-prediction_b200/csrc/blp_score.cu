@@ -43,11 +43,6 @@
 #include <vector>
 
 #include "blp_internal.h"
-
-#ifndef BLP_HUB_TMA
-#define BLP_HUB_TMA 1   // 0: A/B build with the cp.async hub copy (and no async-proxy fences)
-#endif
-
 #include "blp_score_common.cuh"
 #include "blp_score_group.cuh"
 #include "blp_score_light.cuh"
@@ -85,7 +80,6 @@ static_assert(kProbeCap >= kTile && kTile <= 256, "hub[] doubles as the list; pr
 template <int NT>
 __device__ __forceinline__ void tile_scan(TileSmem& ts, int v, int tid, int count) {
     const int lane = tid & 31, warp = tid >> 5;
-#ifndef BLP_NO_SMALL_SCAN
     if (count <= 32) {
         // the common tile (a user's few businesses, a group's 32 pairs) lives in warp 0 alone:
         // one warp scan, one barrier
@@ -107,7 +101,6 @@ __device__ __forceinline__ void tile_scan(TileSmem& ts, int v, int tid, int coun
         __syncthreads();
         return;
     }
-#endif
     int inc = v;
     if (tid < kTile) {
 #pragma unroll
@@ -392,10 +385,7 @@ __device__ unsigned long long g_phase_cycles[16];
 #define BLP_TICK(slot) do {} while (0)
 #endif
 
-#ifndef BLP_THREADS_PER_SM
-#define BLP_THREADS_PER_SM 1024
-#endif
-
+constexpr int kThreadsPerSm = 1024;   // the CTA kernel's occupancy target (__launch_bounds__)
 
 // Descriptor of one work item (group) as the kernel carries it in registers.  The uniform part
 // of the chain  item -> node -> (pair range, row)  is fetched for the NEXT group in two stages
@@ -436,7 +426,7 @@ __device__ __forceinline__ void stage2(const SideArgs& a, GroupRegs& g) {
 }
 
 template <int NT, bool RANGED, bool REC>
-__global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREADS_PER_SM / NT) : 1)
+__global__ void __launch_bounds__(NT, kThreadsPerSm / NT)
     k_score_side(SideArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     unsigned* bm = reinterpret_cast<unsigned*>(smem_raw);
@@ -468,9 +458,7 @@ __global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREA
         const int n4 = a.bm_words >> 2;
         for (int i = tid; i < n4; i += NT) b4[i] = make_uint4(0u, 0u, 0u, 0u);
     }
-#if BLP_HUB_TMA
     fence_async_smem();   // the clear (and the barrier's init) before any bulk copy into the bitmap
-#endif
     __syncthreads();
     GroupRegs cur;
     cur.item = ts.item_next;
@@ -579,7 +567,6 @@ __global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREA
                     // thread and completing on an mbarrier -- no thread spends issue slots or
                     // registers on the 46 KB, and it turns on exactly deg(hub) bits.  The clear
                     // that precedes it was fenced for the async proxy where it was written.
-#if BLP_HUB_TMA
                     if (tid == 0) {
                         const unsigned bytes = (unsigned)a.bm_words * 4u;
                         mbar_expect_tx(&ts.hub_bar, bytes);
@@ -589,20 +576,6 @@ __global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREA
                     first_reg = 1;
                     mbar_wait(&ts.hub_bar, hub_phase);   // every thread: the bytes have landed
                     hub_phase ^= 1u;
-#else
-                    // (A/B build: the Ampere-style copy, 16 bytes per cp.async, every thread issuing)
-                    const uint4* src = h4 + (size_t)ts.hub[0] * hub4;
-                    for (int i = tid; i < n4; i += NT) {
-                        const unsigned dst = (unsigned)__cvta_generic_to_shared(b4 + i);
-                        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src + i)
-                                     : "memory");
-                    }
-                    asm volatile("cp.async.commit_group;" ::: "memory");
-                    if (tid == 0) newbits += ts.cn[0];
-                    first_reg = 1;
-                    asm volatile("cp.async.wait_group 0;" ::: "memory");
-                    (void)hub_phase;
-#endif
                 }
                 if (nhub > first_reg) {
                     const bool fresh = false;   // words are valid (zero or earlier hubs / tiles)
@@ -725,9 +698,7 @@ __global__ void __launch_bounds__(NT, (BLP_THREADS_PER_SM / NT) > 0 ? (BLP_THREA
             uint4* b4 = reinterpret_cast<uint4*>(bm);
             const int n4 = a.bm_words >> 2;
             for (int i = tid; i < n4; i += NT) b4[i] = make_uint4(0u, 0u, 0u, 0u);
-#if BLP_HUB_TMA
             fence_async_smem();   // ... before the next group's bulk copy may land on these words
-#endif
         }
         }   // id-range passes
         if (tid == 0) {   // ordered before the next group's counting by its barriers
@@ -822,12 +793,12 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
         // (round 2, with the hub copy done by TMA: C2 -- 46 KB bitmap -- 700..1000 flat and 3 % better
         // than 1525; C3 / C4 -- 200 KB bitmap, one CTA per SM -- 6667 better than 4500 and 3000)
         int min_deg = (int)std::max<long long>(64, bm_bytes <= 65536 ? bm_bytes / 50 : bm_bytes / 30);
-        if (const char* e = getenv("BLP_HUB_MIN_DEG")) min_deg = atoi(e);   // tuning override
+        if (g->tune.hub_min_deg >= 0) min_deg = g->tune.hub_min_deg;
         // Bitmaps used only by the intersection's probe path start lower: a probe costs about as
         // much as a streamed id, and the path is taken when deg(y) >= kProbeRatio * |hop2(x)|
         // with |hop2(x)| <= kProbeCap, so a bitmap pays off from a few hundred ids on.
         int probe_deg = min_deg > 0 ? std::max(64, min_deg / 3) : 0;
-        if (const char* e = getenv("BLP_PROBE_MIN_DEG")) probe_deg = atoi(e);   // 0 = path off
+        if (g->tune.probe_min_deg >= 0) probe_deg = g->tune.probe_min_deg;   // 0 = path off
         // the slot field needs every first-entry index to fit BLP_ROW_FIRST4_BITS
         const long long mid_entries = us ? g->b_adj_len : g->u_adj_len;
         const bool slots_fit = mid_entries / 4 < (1LL << BLP_ROW_FIRST4_BITS);
@@ -883,8 +854,7 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
                                     cudaMemcpyHostToDevice));
             g->device_bytes += (int64_t)(sizeof(unsigned) * wt.size());
             g->row_slots[side] = true;
-            g->probe_ratio = kProbeRatio;
-            if (const char* e = getenv("BLP_PROBE_RATIO")) g->probe_ratio = std::max(1, atoi(e));
+            g->probe_ratio = g->tune.probe_ratio > 0 ? g->tune.probe_ratio : kProbeRatio;
         }
         int* d_nodes = nullptr;
         const size_t bytes = hubs.size() * (size_t)bm_bytes;
@@ -927,8 +897,7 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
         }
     }
     // which grouping nodes qualify for the warp-per-group kernel (BLP_LIGHT=0 turns it off)
-    const char* le = getenv("BLP_LIGHT");
-    if (!le || atoi(le) != 0) {
+    if (g->tune.light) {
         for (int side = 0; side < 2; ++side) {
             const bool us = side == BLP_SIDE_USER;
             const int n_side = us ? g->n_users : g->n_biz;
@@ -936,8 +905,7 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
             const unsigned long long* g_row = (const unsigned long long*)(us ? g->u_row : g->b_row);
             const unsigned long long* m_row = (const unsigned long long*)(us ? g->b_row : g->u_row);
             BLP_CUDA_TRY(cudaMalloc((void**)&g->light[side], (size_t)n_side));
-            const char* he = getenv("BLP_LIGHT_HUBS");   // BLP_LIGHT_HUBS=0: hub-free groups only
-            const int max_hubs = (g->hubtab_cn[side] && !(he && atoi(he) == 0)) ? 1 : 0;
+            const int max_hubs = (g->hubtab_cn[side] && g->tune.light_hubs) ? 1 : 0;
             k_flag_light<<<(n_side + 255) / 256, 256>>>(
                 n_side, g_row, us ? g->u_adj : g->b_adj,
                 g->xrow[side] ? (const unsigned long long*)g->xrow[side] : m_row, max_hubs,
@@ -1073,8 +1041,7 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
     // no sort: the runs of equal keys are the work items when they average >= 4 pairs.  The
     // decision is taken on the device (k_decide_mode); the kernels of the mode not chosen exit at
     // once, so the call never waits for the host.
-    int force = g->tune.grouping;   // (BLP_GROUPING=runs|sort, read at handle creation)
-    if (!us && force < 0) force = MODE_SORT;   // a per-user list is never grouped by business
+    const int force = us ? -1 : MODE_SORT;   // a per-user list is never grouped by business
     unsigned* cnt = nullptr;
     if (force == MODE_SORT) {   // the mode is certain: the keys pass counts the group sizes as well
         BLP_TRY_SCRATCH(alloc((void**)&cnt, sizeof(unsigned) * (size_t)n_keys));
@@ -1107,39 +1074,37 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
         BLP_TRY_SCRATCH(cudaGetLastError());
         ++launches;
     }
-    if (force != MODE_RUNS) {
-        unsigned* grp_off = nullptr;
-        int2* pg = nullptr;
-        const bool counted = cnt != nullptr;
-        BLP_TRY_SCRATCH(alloc((void**)&inv, sizeof(int) * (size_t)n));
-        // grouped-order result records + gather pass: only when the sort mode is certain (the
-        // business side); a list whose mode is decided on the device writes its outputs directly
-        if (force == MODE_SORT)
-            BLP_TRY_SCRATCH(alloc((void**)&a.rec, sizeof(unsigned long long) * 3 * (size_t)n));
-        if (!counted) BLP_TRY_SCRATCH(alloc((void**)&cnt, sizeof(unsigned) * (size_t)n_keys));
-        BLP_TRY_SCRATCH(alloc((void**)&grp_off, sizeof(unsigned) * (size_t)n_keys));
-        BLP_TRY_SCRATCH(alloc((void**)&pg, sizeof(int2) * (size_t)n));
-        if (!counted) {
-            BLP_TRY_SCRATCH(cudaMemsetAsync(cnt, 0, sizeof(unsigned) * (size_t)n_keys, st));
-            k_group_count<<<gblocks, 256, 0, st>>>(mode, keys, n, cnt);
-            BLP_TRY_SCRATCH(cudaGetLastError());
-            ++launches;
-        }
-        const int n_tiles = (n_keys + kScanTile - 1) / kScanTile;
-        unsigned* tile_sum = nullptr;
-        int* tile_items = nullptr;
-        BLP_TRY_SCRATCH(alloc((void**)&tile_sum, sizeof(unsigned) * (size_t)n_tiles));
-        BLP_TRY_SCRATCH(alloc((void**)&tile_items, sizeof(int) * (size_t)n_tiles));
-        k_group_tile_sums<<<n_tiles, 1024, 0, st>>>(mode, cnt, n_keys, tile_sum, tile_items);
-        k_group_tile_scan<<<1, 1024, 0, st>>>(mode, tile_sum, tile_items, n_tiles, scalars);
-        k_group_tile_apply<<<n_tiles, 1024, 0, st>>>(mode, cnt, n_keys, tile_sum, tile_items, grp_off,
-                                                      item_key, item_start, item_end);
+    unsigned* grp_off = nullptr;
+    int2* pg = nullptr;
+    const bool counted = cnt != nullptr;
+    BLP_TRY_SCRATCH(alloc((void**)&inv, sizeof(int) * (size_t)n));
+    // grouped-order result records + gather pass: only when the sort mode is certain (the
+    // business side); a list whose mode is decided on the device writes its outputs directly
+    if (force == MODE_SORT)
+        BLP_TRY_SCRATCH(alloc((void**)&a.rec, sizeof(unsigned long long) * 3 * (size_t)n));
+    if (!counted) BLP_TRY_SCRATCH(alloc((void**)&cnt, sizeof(unsigned) * (size_t)n_keys));
+    BLP_TRY_SCRATCH(alloc((void**)&grp_off, sizeof(unsigned) * (size_t)n_keys));
+    BLP_TRY_SCRATCH(alloc((void**)&pg, sizeof(int2) * (size_t)n));
+    if (!counted) {
+        BLP_TRY_SCRATCH(cudaMemsetAsync(cnt, 0, sizeof(unsigned) * (size_t)n_keys, st));
+        k_group_count<<<gblocks, 256, 0, st>>>(mode, keys, n, cnt);
         BLP_TRY_SCRATCH(cudaGetLastError());
-        k_group_scatter<<<gblocks, 256, 0, st>>>(mode, keys, gy, n, grp_off, pg, inv);
-        BLP_TRY_SCRATCH(cudaGetLastError());
-        launches += 4;
-        a.pg = pg;
+        ++launches;
     }
+    const int n_tiles = (n_keys + kScanTile - 1) / kScanTile;
+    unsigned* tile_sum = nullptr;
+    int* tile_items = nullptr;
+    BLP_TRY_SCRATCH(alloc((void**)&tile_sum, sizeof(unsigned) * (size_t)n_tiles));
+    BLP_TRY_SCRATCH(alloc((void**)&tile_items, sizeof(int) * (size_t)n_tiles));
+    k_group_tile_sums<<<n_tiles, 1024, 0, st>>>(mode, cnt, n_keys, tile_sum, tile_items);
+    k_group_tile_scan<<<1, 1024, 0, st>>>(mode, tile_sum, tile_items, n_tiles, scalars);
+    k_group_tile_apply<<<n_tiles, 1024, 0, st>>>(mode, cnt, n_keys, tile_sum, tile_items, grp_off,
+                                                  item_key, item_start, item_end);
+    BLP_TRY_SCRATCH(cudaGetLastError());
+    k_group_scatter<<<gblocks, 256, 0, st>>>(mode, keys, gy, n, grp_off, pg, inv);
+    BLP_TRY_SCRATCH(cudaGetLastError());
+    launches += 4;
+    a.pg = pg;
     a.mode = mode;
     a.caller_y = gy;
     a.item_key = item_key;
@@ -1171,9 +1136,7 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
     // ---- persistent scoring grid: as many CTAs per SM as the bitmap allows
     int per_sm = 0, nt = 0, rc = BLP_OK;
     const size_t budget = (size_t)g->max_smem_optin;
-    const int nt_force = g->tune.nt;   // (BLP_NT, read at handle creation)
-    if (nt_force == 256 || nt_force == 512 || nt_force == 1024) nt = nt_force;
-    else if (smem * 4 + 4096 <= budget) nt = 256;
+    if (smem * 4 + 4096 <= budget) nt = 256;
     else if (smem * 2 + 2048 <= budget) nt = 512;
     else nt = 1024;
     const int use_sms = std::max(1, g->sm_count - g->reserve_sms);
@@ -1208,14 +1171,9 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
     // The CTA kernel goes first and the warp-per-group kernel beside it on the handle's side
     // stream: both are persistent work-queue grids, so as the CTA kernel's blocks retire (its
     // groups are few and large, the tail is long) the small warp-per-group blocks fill the SMs.
-    // BLP_LIGHT_STREAM=0 keeps both on the caller's stream.
-    bool light_aside = false;
     if (split) {
-        light_aside = g->side_stream != nullptr && g->tune.light_stream;
-        if (light_aside) {
-            BLP_TRY_SCRATCH(cudaEventRecord(g->ev_fork[side], st));
-            BLP_TRY_SCRATCH(cudaStreamWaitEvent(g->side_stream, g->ev_fork[side], 0));
-        }
+        BLP_TRY_SCRATCH(cudaEventRecord(g->ev_fork[side], st));
+        BLP_TRY_SCRATCH(cudaStreamWaitEvent(g->side_stream, g->ev_fork[side], 0));
     }
     if (nt == 256) {
         if (ranged) BLP_DISPATCH(256, true); else BLP_DISPATCH(256, false);
@@ -1226,17 +1184,17 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
     }
 #undef BLP_DISPATCH
     if (rc == BLP_OK && split) {
-        cudaStream_t lst = light_aside ? g->side_stream : st;
+        cudaStream_t lst = g->side_stream;
         rc = rec_mode ? launch_light<kLightCap, kLightSlots, kLightWarps, true>(g, la, use_sms, lst)
                       : launch_light<kLightCap, kLightSlots, kLightWarps, false>(g, la, use_sms, lst);
         if (rc == BLP_OK) {
             ++launches;
             g->ev_light[side] = cudaEventRecord(g->ev[side][3], lst) == cudaSuccess;
             // join: everything behind this call on the caller's stream waits for the side stream
-            if (light_aside && cudaStreamWaitEvent(st, g->ev[side][3], 0) != cudaSuccess)
+            if (cudaStreamWaitEvent(st, g->ev[side][3], 0) != cudaSuccess)
                 rc = blp::cuda_fail(cudaGetLastError(), "joining the side stream", __FILE__, __LINE__);
         }
-        if (rc != BLP_OK && light_aside) cudaStreamSynchronize(g->side_stream);   // scratch is freed below
+        if (rc != BLP_OK) cudaStreamSynchronize(lst);   // scratch is freed below
     }
     if (rc == BLP_OK && a.rec) {
         k_unpermute<<<gblocks, 256, 0, st>>>(a.mode, a.rec, inv, n, a.cn, a.uni, a.jac, a.aa);

@@ -8,14 +8,8 @@
 namespace blp {
 
 
-#ifndef BLP_TILE
-#define BLP_TILE 256
-#endif
-constexpr int kTile = BLP_TILE;   // adjacency lists per scheduling tile (<= threads per CTA)
-#ifndef BLP_CHUNK_V4
-#define BLP_CHUNK_V4 128
-#endif
-constexpr int kChunkV4 = BLP_CHUNK_V4;   // int4 loads per chunk (at most 4 per lane): 512 ids
+constexpr int kTile = 256;      // adjacency lists per scheduling tile (<= threads per CTA)
+constexpr int kChunkV4 = 128;   // int4 loads per chunk (at most 4 per lane): 512 ids
 constexpr unsigned kFull = 0xffffffffu;
 
 struct SideArgs {
@@ -84,30 +78,18 @@ struct SideArgs {
 // The graph (adjacency, weights, hub bitmaps, row descriptors) is what every group re-reads; the
 // pair ids, the per-call scratch and the result columns stream through once.  Graph loads carry an
 // L2 evict_last policy, the streams use evict-first loads / stores (ld/st.global.cs), so that the
-// 0.5 GB of results per step do not push the graph out of L2 (BLP_L2_HINTS=0 compiles both away).
-#ifndef BLP_L2_HINTS
-#define BLP_L2_HINTS 1
-#endif
-
+// 0.5 GB of results per step do not push the graph out of L2.
 __device__ __forceinline__ unsigned long long l2_keep_policy() {
     unsigned long long pol = 0ull;
-#if BLP_L2_HINTS
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-#endif
     return pol;
 }
 
 __device__ __forceinline__ int4 ldg_stream(const int4* p, unsigned long long pol) {
     int4 r;
-#if BLP_L2_HINTS
     asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.s32 {%0,%1,%2,%3}, [%4], %5;"
                  : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
                  : "l"(p), "l"(pol));
-#else
-    asm volatile("ld.global.nc.L1::no_allocate.v4.s32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
-                 : "l"(p));
-#endif
     return r;
 }
 
@@ -123,56 +105,34 @@ __device__ __forceinline__ int row_slot1(unsigned long long row) {
 
 __device__ __forceinline__ uint4 ldg_stream_u(const uint4* p, unsigned long long pol) {
     uint4 r;
-#if BLP_L2_HINTS
     asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
                  : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
                  : "l"(p), "l"(pol));
-#else
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
-                 : "l"(p));
-#endif
     return r;
 }
 
 // graph data through the read-only path with the keep-in-L2 policy (L1 allocation as usual)
 __device__ __forceinline__ uint4 ldg_keep(const uint4* p, unsigned long long pol) {
-#if BLP_L2_HINTS
     uint4 r;
     asm volatile("ld.global.nc.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
                  : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
                  : "l"(p), "l"(pol));
     return r;
-#else
-    return __ldg(p);
-#endif
 }
 __device__ __forceinline__ unsigned ldg_keep(const unsigned* p, unsigned long long pol) {
-#if BLP_L2_HINTS
     unsigned r;
     asm volatile("ld.global.nc.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(pol));
     return r;
-#else
-    return __ldg(p);
-#endif
 }
 
 // streaming (evict-first) accessors for data that passes through once
 template <typename T>
 __device__ __forceinline__ void st_stream(T* p, T v) {
-#if BLP_L2_HINTS
     __stcs(p, v);
-#else
-    *p = v;
-#endif
 }
 template <typename T>
 __device__ __forceinline__ T ld_once(const T* p) {
-#if BLP_L2_HINTS
     return __ldcs(p);
-#else
-    return *p;
-#endif
 }
 
 // ---- TMA bulk copy + mbarrier (sm_90+; the hub-bitmap copy of k_score_side) --------------------

@@ -55,7 +55,7 @@ __global__ void k_count_runs(const int* __restrict__ keys, long long n, unsigned
 }
 
 // Grouping mode, decided on the device so that the call never waits for the host:
-// runs are used when they average >= 4 pairs (BLP_GROUPING=runs/sort forces a mode).
+// runs are used when they average >= 4 pairs (the business side forces sort mode).
 __global__ void k_decide_mode(const unsigned* __restrict__ n_runs, long long n, int force,
                               int* __restrict__ mode) {
     *mode = force >= 0 ? force : (((long long)*n_runs * 4 <= n) ? MODE_RUNS : MODE_SORT);

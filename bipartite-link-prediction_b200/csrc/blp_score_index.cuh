@@ -19,10 +19,6 @@
 #include "blp_score_common.cuh"
 #include "blp_score_group.cuh"
 
-#ifndef BLP_BIZ_INDEX_KEEP
-#define BLP_BIZ_INDEX_KEEP 1   // 0: index-row loads without the evict_last policy (A/B build)
-#endif
-
 namespace blp {
 
 constexpr int kIndexBuildThreads = 512;
@@ -99,20 +95,11 @@ __global__ void __launch_bounds__(kIndexBuildThreads) k_build_biz_index(
     }
 }
 
-__device__ __forceinline__ unsigned index_word(const unsigned* p, unsigned long long pol) {
-#if BLP_BIZ_INDEX_KEEP
-    return ldg_keep(p, pol);
-#else
-    (void)pol;
-    return __ldg(p);
-#endif
-}
-
 // four ids of N(u) (padding: the sentinel n_biz, whose bit is never set, weight 0) against row b
 __device__ __forceinline__ void index_test4(const unsigned* row, int4 v, uint4 wt, unsigned& cnt,
                                             unsigned long long& acc, unsigned long long pol) {
-    const unsigned w0 = index_word(row + (v.x >> 5), pol), w1 = index_word(row + (v.y >> 5), pol);
-    const unsigned w2 = index_word(row + (v.z >> 5), pol), w3 = index_word(row + (v.w >> 5), pol);
+    const unsigned w0 = ldg_keep(row + (v.x >> 5), pol), w1 = ldg_keep(row + (v.y >> 5), pol);
+    const unsigned w2 = ldg_keep(row + (v.z >> 5), pol), w3 = ldg_keep(row + (v.w >> 5), pol);
     const unsigned h0 = (w0 >> (v.x & 31)) & 1u, h1 = (w1 >> (v.y & 31)) & 1u;
     const unsigned h2 = (w2 >> (v.z & 31)) & 1u, h3 = (w3 >> (v.w & 31)) & 1u;
     cnt += h0 + h1 + h2 + h3;

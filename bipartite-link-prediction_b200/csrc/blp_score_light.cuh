@@ -28,13 +28,8 @@ namespace blp {
 // (A larger-table "medium" instance with 8 groups in flight per SM was measured and is slower than
 // the CTA kernel: one warp streaming a hub partner's list is too slow.)
 // ---------------------------------------------------------------------------------------------
-#ifndef BLP_LIGHT_CAP
-#define BLP_LIGHT_CAP 512
-#endif
-#ifndef BLP_LIGHT_MIN_CTAS
-#define BLP_LIGHT_MIN_CTAS 4
-#endif
-constexpr int kLightCap = BLP_LIGHT_CAP, kLightSlots = 1024, kLightWarps = 8;
+constexpr int kLightCap = 512, kLightSlots = 1024, kLightWarps = 8;
+constexpr int kLightMinCtas = 4;   // __launch_bounds__ occupancy target of k_score_light
 constexpr int kLightEmpty = -1;
 
 template <int CAP, int SLOTS>
@@ -201,7 +196,7 @@ __device__ __forceinline__ void light_stage_e(const SideArgs& a, LightRegs& g) {
 }
 
 template <int CAP, int SLOTS, int WARPS, bool REC>
-__global__ void __launch_bounds__(WARPS * 32, BLP_LIGHT_MIN_CTAS) k_score_light(SideArgs a) {
+__global__ void __launch_bounds__(WARPS * 32, kLightMinCtas) k_score_light(SideArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     typedef LightSmem<CAP, SLOTS> Smem;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;

@@ -426,7 +426,6 @@ class HostSession(object):
     library.  By default the columns are the seven outputs the reference leaves on the host
     (similarity.py:61,106 + PA: 48 B per pair); the two union sizes are extra (``columns='all'``,
     56 B) -- the link is the bottleneck of this call, so bytes that nobody reads stay on the device.
-    `score_pinned_py` drives the same pipeline from Python.
     """
 
     ALL_KEYS = ('u_cn', 'u_union', 'u_jaccard', 'u_adamic', 'b_cn', 'b_union', 'b_jaccard',
@@ -451,7 +450,6 @@ class HostSession(object):
         self.h_out = {}
         for k in self.KEYS:
             self.h_out[k] = torch.empty(n, dtype=self.DTYPES[k.split('_')[-1]]).pin_memory()
-        self.d_out = None          # device staging of score_pinned_py, made on first use
         self.h2d_bytes_per_pair = 8
         self.d2h_bytes_per_pair = sum(self.h_out[k].element_size() for k in self.KEYS)
 
@@ -482,14 +480,6 @@ class HostSession(object):
                 'what': 'pinned copies timed alone on this box; d2h_floor_ms = the %d result bytes '
                         'of one step at that rate' % d2h_bytes}
 
-    def _device_staging(self):
-        if self.d_out is None:
-            dev, n = self.g.device, self.n_max
-            self.d_u = torch.empty(n, dtype=torch.int32, device=dev)
-            self.d_b = torch.empty(n, dtype=torch.int32, device=dev)
-            self.d_out = {k: torch.empty(n, dtype=self.h_out[k].dtype, device=dev) for k in self.KEYS}
-            self.copy_stream = torch.cuda.Stream(device=dev)
-
     def pinned_inputs(self, n):
         """Numpy views of the pinned pair buffers, for callers that fill them in place."""
         return self.h_u[:n].numpy(), self.h_b[:n].numpy()
@@ -517,91 +507,4 @@ class HostSession(object):
         _lib.check(lib.blp_score_pairs_host(self.g._h, self.h_u.data_ptr(), self.h_b.data_ptr(), n,
                                             *outs, int(user_chunks), int(lead_chunks),
                                             int(biz_chunks)), 'blp_score_pairs_host')
-        return {k: self.h_out[k][:n].numpy() for k in self.KEYS}
-
-    def score_pinned_py(self, n, user_chunks=4, lead_chunks=1, biz_chunks=2):
-        """The same pipeline driven from Python over blp_score_pairs (kept for comparison: the
-        host-side cost of ~100 launches and copies per step shows up as GPU idle time).
-
-        The device scores a step faster than the link can carry its results back (56 B per pair
-        over PCIe: 560 MB at ~57 GB/s is 9.8 ms for the C2 step, the kernels need ~8 ms), so the
-        pipeline is arranged around the copy-back engine: start it as early as possible and never
-        let it idle.  The pair ids of the first `lead_chunks` user-side slices go up first and are
-        scored at once (their results start the D2H engine), the rest of the ids follow on a
-        separate upload stream; then the business side and the remaining user-side slices take
-        turns -- the business side in `biz_chunks` slices, so that no single launch leaves the
-        engine without work -- each slice's copy-back overlapping the next slice's scoring.
-        """
-        n = int(n)
-        if n > self.n_max:
-            raise ValueError('pair count %d exceeds the session capacity %d' % (n, self.n_max))
-        self._device_staging()
-        g, dev = self.g, self.g.device
-        ukeys = [k for k in self.KEYS if not k.startswith('b_')]
-        bkeys = [k for k in self.KEYS if k.startswith('b_')]
-        with torch.cuda.device(dev):
-            main = torch.cuda.current_stream(dev)
-            copy = self.copy_stream
-            if getattr(self, 'up_stream', None) is None:
-                self.up_stream = torch.cuda.Stream(device=dev)
-            up = self.up_stream
-            du, db = self.d_u[:n], self.d_b[:n]
-            chunks = max(1, min(int(user_chunks), n // 65536 or 1))
-            bounds = [(n * c) // chunks for c in range(chunks + 1)]
-            lead = max(0, min(int(lead_chunks), chunks - 1))
-            bchunks = max(1, min(int(biz_chunks), n // 65536 or 1))
-            bbounds = [(n * c) // bchunks for c in range(bchunks + 1)]
-            head = bounds[lead]
-            # upload: the head on the main stream, the rest beside it
-            if head:
-                du[:head].copy_(self.h_u[:head], non_blocking=True)
-                db[:head].copy_(self.h_b[:head], non_blocking=True)
-            up.wait_stream(main)
-            with torch.cuda.stream(up):
-                du[head:].copy_(self.h_u[head:n], non_blocking=True)
-                db[head:].copy_(self.h_b[head:n], non_blocking=True)
-                ev_up = torch.cuda.Event()
-                ev_up.record(up)
-
-            def copy_back(names, lo, hi):
-                ev = torch.cuda.Event()
-                ev.record(main)
-                with torch.cuda.stream(copy):
-                    copy.wait_event(ev)
-                    for k in names:
-                        self.h_out[k][lo:hi].copy_(self.d_out[k][lo:hi], non_blocking=True)
-
-            def user_slice(c):
-                lo, hi = bounds[c], bounds[c + 1]
-                if hi <= lo:
-                    return
-                ou = {(k[2:] if k.startswith('u_') else k): self.d_out[k][lo:hi] for k in ukeys}
-                g.score_side(_lib.SIDE_USER, du[lo:hi], db[lo:hi], want_pa=True, out=ou)
-                copy_back(ukeys, lo, hi)
-
-            def biz_slice(c):
-                lo, hi = bbounds[c], bbounds[c + 1]
-                if hi <= lo:
-                    return
-                ob = {k[2:]: self.d_out[k][lo:hi] for k in bkeys}
-                g.score_side(_lib.SIDE_BUSINESS, du[lo:hi], db[lo:hi], out=ob)
-                copy_back(bkeys, lo, hi)
-
-            for c in range(lead):
-                user_slice(c)
-            main.wait_event(ev_up)
-            # the remaining user slices with the business slices spread evenly between them
-            rest = list(range(lead, chunks))
-            per = -(-len(rest) // bchunks) if rest else 0
-            bi = 0
-            for i, c in enumerate(rest):
-                if per and i % per == 0 and bi < bchunks:
-                    biz_slice(bi)
-                    bi += 1
-                user_slice(c)
-            while bi < bchunks:
-                biz_slice(bi)
-                bi += 1
-            main.wait_stream(copy)
-            main.synchronize()
         return {k: self.h_out[k][:n].numpy() for k in self.KEYS}

@@ -6,6 +6,11 @@ inside both, the probe / table path for partners that have a bitmap.  Which one 
 depends on thresholds read at graph creation (BLP_* tuning variables).  These tests force small
 graphs through every combination and require (a) bit-identical outputs across the combinations and
 (b) agreement with the C oracle.
+
+A handle that fits a business index scores the business side with it, so every combination but
+the library defaults also sets BLP_BIZ_INDEX=0: the business side then takes the grouped path (sort
+mode, result records and un-permute, the warp-per-group kernel and hub tables), the only one for
+graphs too large for an index and for ranged handles, and the defaults compare the index against it.
 """
 import numpy as np
 import pytest
@@ -15,30 +20,37 @@ from test_gpu_parity import check_against, mods  # noqa: F401
 
 pytestmark = pytest.mark.gpu
 
-TUNING = ('BLP_LIGHT', 'BLP_LIGHT_HUBS', 'BLP_PROBE_MIN_DEG', 'BLP_PROBE_RATIO', 'BLP_HUB_MIN_DEG')
+TUNING = ('BLP_LIGHT', 'BLP_LIGHT_HUBS', 'BLP_PROBE_MIN_DEG', 'BLP_PROBE_RATIO', 'BLP_HUB_MIN_DEG',
+          'BLP_BIZ_INDEX')
+GROUPED = dict(BLP_BIZ_INDEX='0')   # the business side without the index
 
 # (light kernel, one-hub groups in it, probe bitmaps from this degree on [0 = off], ratio, OR-hub degree)
 COMBOS = [
-    dict(BLP_LIGHT='0', BLP_PROBE_MIN_DEG='0', BLP_HUB_MIN_DEG='0'),      # CTA kernel, lists only
-    dict(BLP_LIGHT='0', BLP_PROBE_MIN_DEG='0', BLP_HUB_MIN_DEG='150'),    # + hub bitmaps
-    dict(BLP_LIGHT='0', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='150', BLP_PROBE_RATIO='1'),
-    dict(BLP_LIGHT='1', BLP_PROBE_MIN_DEG='0', BLP_HUB_MIN_DEG='150'),    # warp kernel, no probing
-    dict(BLP_LIGHT='1', BLP_LIGHT_HUBS='0', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='150'),
-    dict(BLP_LIGHT='1', BLP_LIGHT_HUBS='1', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='150',
+    dict(GROUPED, BLP_LIGHT='0', BLP_PROBE_MIN_DEG='0', BLP_HUB_MIN_DEG='0'),     # CTA kernel, lists only
+    dict(GROUPED, BLP_LIGHT='0', BLP_PROBE_MIN_DEG='0', BLP_HUB_MIN_DEG='150'),   # + hub bitmaps
+    dict(GROUPED, BLP_LIGHT='0', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='150', BLP_PROBE_RATIO='1'),
+    dict(GROUPED, BLP_LIGHT='1', BLP_PROBE_MIN_DEG='0', BLP_HUB_MIN_DEG='150'),   # warp kernel, no probing
+    dict(GROUPED, BLP_LIGHT='1', BLP_LIGHT_HUBS='0', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='150'),
+    dict(GROUPED, BLP_LIGHT='1', BLP_LIGHT_HUBS='1', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='150',
          BLP_PROBE_RATIO='1'),
-    dict(BLP_LIGHT='1', BLP_LIGHT_HUBS='1', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='64',
+    dict(GROUPED, BLP_LIGHT='1', BLP_LIGHT_HUBS='1', BLP_PROBE_MIN_DEG='64', BLP_HUB_MIN_DEG='64',
          BLP_PROBE_RATIO='4'),
     dict(),                                                                  # library defaults
 ]
 
 
 def score_with(monkeypatch, graph, env, n_users, n_biz, eu, eb, pu, pv):
+    """Scores both sides on a handle created under exactly `env` and checks which path its
+    business side took: grouped under BLP_BIZ_INDEX=0, else the index (these graphs are small)."""
+    lib = pkg('_lib')
     for k in TUNING:
         monkeypatch.delenv(k, raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     G = graph.BipartiteGraph(n_users, n_biz, eu, eb)
     out = G.score_pairs_host(pu, pv, want_hop2=True)
+    want_path = lib.PATH_GROUPED if env.get('BLP_BIZ_INDEX') == '0' else lib.PATH_BIZ_INDEX
+    assert G.score_stats(lib.SIDE_BUSINESS)['path'] == want_path, env
     info = G.info()
     G.close()
     return out, info
@@ -86,7 +98,7 @@ def test_all_paths_agree(mods, monkeypatch, seed, n_users, n_biz, n_rev, k, alph
 
 def test_business_side_light_groups_and_unsorted_input(mods, monkeypatch):
     """Pairs in random order (sort-mode grouping, record + un-permute epilogue) through the
-    warp-per-group kernel on both sides."""
+    warp-per-group kernel on both sides (the business side without the index)."""
     from oracle import c_oracle
     graph, synth = mods
     n_users, n_biz = 8000, 3000
@@ -95,7 +107,7 @@ def test_business_side_light_groups_and_unsorted_input(mods, monkeypatch):
     perm = np.random.default_rng(3).permutation(pu.size)
     pu, pv = pu[perm].copy(), pv[perm].copy()
     want = c_oracle.score_pair_arrays(n_users, n_biz, eu, eb, pu, pv)
-    for env in (dict(BLP_HUB_MIN_DEG='100', BLP_PROBE_MIN_DEG='64'), dict(BLP_LIGHT='0')):
+    for env in (dict(GROUPED, BLP_HUB_MIN_DEG='100', BLP_PROBE_MIN_DEG='64'), dict(GROUPED, BLP_LIGHT='0')):
         got, _ = score_with(monkeypatch, graph, env, n_users, n_biz, eu, eb, pu, pv)
         check_against(got, want, pu.size)
 
@@ -121,9 +133,9 @@ def test_light_group_corner_cases(mods, monkeypatch):
     pu = np.repeat(np.array(users, np.int32), n_biz)
     pv = np.tile(np.arange(n_biz, dtype=np.int32), len(users))
     want = c_oracle.score_pair_arrays(n_users, n_biz, eu, eb, pu, pv)
-    for env in (dict(BLP_HUB_MIN_DEG='200', BLP_PROBE_MIN_DEG='64', BLP_PROBE_RATIO='1'),
-                dict(BLP_HUB_MIN_DEG='64', BLP_PROBE_MIN_DEG='64'),
-                dict(BLP_LIGHT='0', BLP_HUB_MIN_DEG='200', BLP_PROBE_MIN_DEG='64'),
+    for env in (dict(GROUPED, BLP_HUB_MIN_DEG='200', BLP_PROBE_MIN_DEG='64', BLP_PROBE_RATIO='1'),
+                dict(GROUPED, BLP_HUB_MIN_DEG='64', BLP_PROBE_MIN_DEG='64'),
+                dict(GROUPED, BLP_LIGHT='0', BLP_HUB_MIN_DEG='200', BLP_PROBE_MIN_DEG='64'),
                 dict()):
         got, _ = score_with(monkeypatch, graph, env, n_users, n_biz, eu, eb, pu, pv)
         check_against(got, want, pu.size)

@@ -1,5 +1,5 @@
 """Developer tool: per-phase cycle shares of the CTA kernel (k_score_side) from a BLP_PHASE_TIMING
-build of the SAME sources (tools/build_variants.py phase="-DBLP_PHASE_TIMING").  Thread 0 of every
+build of the SAME sources (compiled into variants/libblp_phase.so on first use).  Thread 0 of every
 CTA adds clock64() deltas at the phase boundaries to a global table; the shares are of CTA-resident
 cycles.  Writes gpurun_out/phase_<config>.json (copy to profiles/r02_phase_shares.json for bench.py).
 usage: phase_time.py [CONFIG] [n_pairs]"""

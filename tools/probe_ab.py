@@ -24,13 +24,10 @@ flush = torch.empty(256 << 20, dtype=torch.uint8, device='cuda')
 base = None
 for s in settings.split(','):
     min_deg, ratio, light, medium = s.split(':')[:4]
-    extra = s.split(':')[4:]          # optional: hub_min_deg, threads per CTA of the CTA kernel
-    for k in ('BLP_HUB_MIN_DEG', 'BLP_NT'):
-        os.environ.pop(k, None)
-    if len(extra) > 0 and int(extra[0]) > 0:
+    extra = s.split(':')[4:5]         # optional: hub_min_deg
+    os.environ.pop('BLP_HUB_MIN_DEG', None)
+    if extra and int(extra[0]) > 0:
         os.environ['BLP_HUB_MIN_DEG'] = extra[0]
-    if len(extra) > 1 and int(extra[1]) > 0:
-        os.environ['BLP_NT'] = extra[1]
     os.environ['BLP_LIGHT'] = light
     os.environ['BLP_LIGHT_HUBS'] = medium
     os.environ.pop('BLP_PROBE_MIN_DEG', None)
