@@ -1,14 +1,12 @@
 // Graph construction on the device (SURVEY.md section 8f, rank 1: the step in front of the path).
-// Replaces snap.LoadEdgeList(snap.PUNGraph, graph_file, 0, 1) (similarity.py:16) for callers whose
-// edge arrays already live in HBM:
+// Replaces snap.LoadEdgeList(snap.PUNGraph, graph_file, 0, 1) (similarity.py:16).  Both create
+// functions run the one builder here: blp_graph_create_device on edge arrays already in HBM,
+// blp_graph_create after copying its host arrays to the device.
 //
 //   keys (u << 32 | b)  --LSD radix sort, 8 bits per pass, only the bits in use-->  sorted keys
 //   --adjacent-difference flags + scan-->  distinct edges (duplicates collapse, SNAP TUNGraph)
 //   --degrees, padded row offsets (scan)-->  user rows (from the sorted order), business rows
 //   (atomic cursors)  --bank striping, sentinels, per-entry weights, row descriptors.
-//
-// Row order inside a row differs from the host builder's (nothing depends on it); every score
-// is identical, which tests/test_gpu_build.py checks.
 #include <algorithm>
 #include <climits>
 #include <cstdio>
@@ -291,8 +289,13 @@ __global__ void k_row_descriptors(const unsigned long long* __restrict__ off,
     }
 }
 
-// Bank striping of one row per warp (see blp_graph.cu: bank_stripe_row for the why).  The ids are
-// first bucketed by bank into `tmp`; id number r of bank b then goes to sequence position
+// Bank striping, one row per warp.  The kernels probe a shared-memory bitmap with one 32-bit load
+// per id; word id>>5 lives in bank (id>>5)&31, so 32 random ids cost ~3 wavefronts instead of 1.
+// Nothing in the algorithm needs a row in ascending order, so every row longer than the sub-warp
+// path (16 ids) is permuted once here: the 32 ids that ONE load instruction touches (lane l reads
+// component q of the int4 at index 32*block + l, i.e. slots 128*block + 4*l + q) are drawn from
+// 32 different banks for as long as every bank still has ids left.  The ids are first bucketed by
+// bank into `tmp`; id number r of bank b then goes to sequence position
 //   e = sum_b' min(cnt[b'], r) + #{b' < b : cnt[b'] > r}
 // (wave r holds one id of every bank that still has ids), and sequence position e of a full
 // 128-slot block sits at slot 4*(e%32) + (e%128)/32 of that block -- the 32 ids one load
@@ -524,15 +527,14 @@ int parse_tile_counts(const char* text, long long n_bytes, cudaStream_t st, unsi
 
 // ------------------------------------------------------------------------------------ id ranges
 // One warp per row of a ranged side's middle adjacency: count the ids of every id range, write the
-// exclusive prefix to seg_off[row][0..R] and -- unless the row is known to ascend already -- move
-// the ids so that range 0's come first, then range 1's, ... (order inside a range is free).  The
-// padding at the row's tail (sentinel ids) is not touched and belongs to no segment.
+// exclusive prefix to seg_off[row][0..R] and move the ids so that range 0's come first, then range
+// 1's, ... (order inside a range is free).  The padding at the row's tail (sentinel ids) is not
+// touched and belongs to no segment.
 namespace {
 __global__ void __launch_bounds__(256) k_range_segments(const unsigned long long* __restrict__ row_desc,
                                                         int n_rows, int* __restrict__ adj,
                                                         int* __restrict__ tmp, int range_bits, int n_ranges,
-                                                        int reorder, int* __restrict__ seg_off,
-                                                        int* __restrict__ next_row) {
+                                                        int* __restrict__ seg_off, int* __restrict__ next_row) {
     __shared__ int s_cnt[8][kMaxRanges + 1], s_cur[8][kMaxRanges + 1];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (;;) {
@@ -558,7 +560,7 @@ __global__ void __launch_bounds__(256) k_range_segments(const unsigned long long
         }
         __syncwarp();
         for (int k = lane; k <= n_ranges; k += 32) seg_off[(size_t)r * (n_ranges + 1) + k] = s_cnt[warp][k];
-        if (reorder && len > 1) {
+        if (len > 1) {
             int* t = tmp + first;
             for (int i = lane; i < len; i += 32) {
                 const int id = row[i];
@@ -572,7 +574,7 @@ __global__ void __launch_bounds__(256) k_range_segments(const unsigned long long
 }
 }  // namespace
 
-int build_range_segments(blp_graph* g, bool reorder, int* tmp, cudaStream_t st) {
+int build_range_segments(blp_graph* g, int* tmp, cudaStream_t st) {
     for (int side = 0; side < 2; ++side) {
         const int R = g->n_ranges[side];
         if (R <= 1) continue;
@@ -590,17 +592,11 @@ int build_range_segments(blp_graph* g, bool reorder, int* tmp, cudaStream_t st) 
         int* counter = nullptr;
         BLP_CUDA_TRY(cudaMalloc((void**)&counter, sizeof(int)));
         BLP_CUDA_TRY(cudaMemsetAsync(counter, 0, sizeof(int), st));
-        int* scratch = tmp;
-        if (reorder && !scratch) {
-            const long long len = us ? g->b_adj_len : g->u_adj_len;
-            BLP_CUDA_TRY(cudaMalloc((void**)&scratch, sizeof(int) * (size_t)std::max<long long>(len, 1)));
-        }
-        k_range_segments<<<g->sm_count * 4, 256, 0, st>>>(rows, n_mid, adj, scratch, g->range_words[side] * 32,
-                                                          R, reorder ? 1 : 0, g->seg_off[side], counter);
+        k_range_segments<<<g->sm_count * 4, 256, 0, st>>>(rows, n_mid, adj, tmp, g->range_words[side] * 32,
+                                                          R, g->seg_off[side], counter);
         cudaError_t e = cudaGetLastError();
         if (e == cudaSuccess) e = cudaStreamSynchronize(st);
         cudaFree(counter);
-        if (scratch != tmp) cudaFree(scratch);
         if (e != cudaSuccess) return cuda_fail(e, "k_range_segments", __FILE__, __LINE__);
     }
     return BLP_OK;
@@ -683,28 +679,36 @@ extern "C" int blp_edge_list_parse(const char* text_dev, int64_t n_bytes, int64_
     return BLP_OK;
 }
 
-extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n_edges,
-                                       const int32_t* edge_u_dev, const int32_t* edge_b_dev,
-                                       int device, void* stream, blp_graph** out) {
-    using namespace blp;
+namespace blp {
+namespace {
+// The argument checks of both create functions, in this order and before any CUDA call but the
+// device count.
+int check_create_args(const char* api, int32_t n_users, int32_t n_biz, int64_t n_edges,
+                      const int32_t* edge_u, const int32_t* edge_b, int device, blp_graph** out) {
     if (!out) {
-        set_error("blp_graph_create_device: out is null");
+        set_error(std::string(api) + ": out is null");
         return BLP_ERR_INVALID;
     }
     *out = nullptr;
-    if (n_users <= 0 || n_biz <= 0 || n_edges < 0 || (n_edges > 0 && (!edge_u_dev || !edge_b_dev))) {
-        set_error("blp_graph_create_device: need n_users>0, n_biz>0, n_edges>=0 and edge arrays");
+    if (n_users <= 0 || n_biz <= 0 || n_edges < 0 || (n_edges > 0 && (!edge_u || !edge_b))) {
+        set_error(std::string(api) + ": need n_users>0, n_biz>0, n_edges>=0 and edge arrays");
         return BLP_ERR_INVALID;
     }
     int ndev = 0;
     int rc = blp_device_count(&ndev);
     if (rc != BLP_OK) return rc;
     if (device < 0 || device >= ndev) {
-        set_error("blp_graph_create_device: device index out of range");
+        set_error(std::string(api) + ": device index out of range");
         return BLP_ERR_INVALID;
     }
-    BLP_ON_DEVICE(device);
-    cudaStream_t st = (cudaStream_t)stream;
+    return BLP_OK;
+}
+
+// The graph builder behind both create functions: edge arrays in device memory, run on `st` of
+// the current device.  `api` names the entry point in error messages.
+int build_graph(const char* api, int32_t n_users, int32_t n_biz, int64_t n_edges,
+                const int32_t* edge_u_dev, const int32_t* edge_b_dev, int device, cudaStream_t st,
+                blp_graph** out) {
     const long long n = n_edges;
     int sm_query = 0;
     if (cudaDeviceGetAttribute(&sm_query, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sm_query <= 0)
@@ -713,7 +717,7 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
 
     blp_graph* g = new (std::nothrow) blp_graph();
     if (!g) {
-        set_error("blp_graph_create_device: host allocation failed");
+        set_error(std::string(api) + ": host allocation failed");
         return BLP_ERR_OOM;
     }
     g->n_users = n_users;
@@ -763,8 +767,8 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
     BLP_TRY_B(cudaStreamSynchronize(st));
     if (bad_host != INT_MAX) {
         char buf[160];
-        snprintf(buf, sizeof(buf), "blp_graph_create_device: edge %d outside [0,%d) x [0,%d)",
-                 bad_host, n_users, n_biz);
+        snprintf(buf, sizeof(buf), "%s: edge %d outside [0,%d) x [0,%d)", api, bad_host, n_users,
+                 n_biz);
         set_error(buf);
         return fail(BLP_ERR_RANGE);
     }
@@ -823,7 +827,7 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
     if (u_len / 4 >= (1ull << BLP_ROW_FIRST4_BITS) || b_len / 4 >= (1ull << BLP_ROW_FIRST4_BITS) ||
         g->max_udeg >= (1 << 24) ||
         g->max_bdeg >= (1 << 24)) {
-        set_error("blp_graph_create_device: graph too large for the packed row descriptors");
+        set_error(std::string(api) + ": graph too large for the packed row descriptors");
         return fail(BLP_ERR_UNSUPPORTED);
     }
 
@@ -867,7 +871,7 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
     if (g->n_ranges[0] == 1)
         k_bank_stripe<<<g->sm_count * 4, 256, 0, st>>>(b_off, b_deg, n_biz, g->b_adj, tmp, next_row + 1);
     BLP_TRY_B(cudaGetLastError());
-    BLP_RC_B(build_range_segments(g, /*reorder=*/true, tmp, st));
+    BLP_RC_B(build_range_segments(g, tmp, st));
 
     // ---- per-entry weights from a host-evaluated 1/ln(d) table
     {
@@ -887,10 +891,49 @@ extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n
     scratch.clear();
     scan.release();
     BLP_TRY_B(cudaStreamSynchronize(st));
-    rc = build_hub_bitmaps(g, hu.data(), hb.data());
+    const int rc = build_hub_bitmaps(g, hu.data(), hb.data());
     if (rc != BLP_OK) return fail(rc);
 #undef BLP_TRY_B
 #undef BLP_RC_B
     *out = g;
     return BLP_OK;
+}
+}  // namespace
+}  // namespace blp
+
+extern "C" int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n_edges,
+                                       const int32_t* edge_u_dev, const int32_t* edge_b_dev,
+                                       int device, void* stream, blp_graph** out) {
+    const char* api = "blp_graph_create_device";
+    int rc = blp::check_create_args(api, n_users, n_biz, n_edges, edge_u_dev, edge_b_dev, device, out);
+    if (rc != BLP_OK) return rc;
+    BLP_ON_DEVICE(device);
+    return blp::build_graph(api, n_users, n_biz, n_edges, edge_u_dev, edge_b_dev, device,
+                            (cudaStream_t)stream, out);
+}
+
+extern "C" int blp_graph_create(int32_t n_users, int32_t n_biz, int64_t n_edges,
+                                const int32_t* edge_u, const int32_t* edge_b, int device,
+                                blp_graph** out) {
+    const char* api = "blp_graph_create";
+    int rc = blp::check_create_args(api, n_users, n_biz, n_edges, edge_u, edge_b, device, out);
+    if (rc != BLP_OK) return rc;
+    BLP_ON_DEVICE(device);
+    // staged and built on the legacy default stream, so the build follows the caller's earlier work
+    // on every blocking stream of the device
+    const cudaStream_t st = cudaStreamLegacy;
+    const size_t bytes = sizeof(int32_t) * (size_t)n_edges;
+    int32_t *eu = nullptr, *eb = nullptr;
+    cudaError_t e = cudaSuccess;
+    if (n_edges > 0) {
+        e = blp::scratch_alloc((void**)&eu, bytes, st);
+        if (e == cudaSuccess) e = blp::scratch_alloc((void**)&eb, bytes, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(eu, edge_u, bytes, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(eb, edge_b, bytes, cudaMemcpyHostToDevice, st);
+    }
+    rc = e == cudaSuccess ? blp::build_graph(api, n_users, n_biz, n_edges, eu, eb, device, st, out)
+                          : blp::cuda_fail(e, "staging the edge arrays", __FILE__, __LINE__);
+    if (eu) cudaFreeAsync(eu, st);
+    if (eb) cudaFreeAsync(eb, st);
+    return rc;
 }

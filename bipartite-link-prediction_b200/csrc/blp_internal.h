@@ -58,9 +58,9 @@ struct blp_graph {
     // Both CSR directions.  Every row is padded AT ITS TAIL to a multiple of four ids with the
     // sentinel n_biz (user rows) / n_users (business rows), so every row starts 16-byte aligned and
     // is read with 128-bit loads without a tail; the first deg(row) entries are the real ids
-    // (blp_hop3 and the light-kernel prefetch rely on that).  Rows of <= 16 ids ascend; longer rows
-    // are bank-striped (a permutation of the row, see bank_stripe_row) -- nothing may assume a
-    // sorted row, so no binary search over rows.
+    // (blp_hop3 and the light-kernel prefetch rely on that).  Nothing else about the order inside
+    // a row may be assumed (business rows are filled through atomic cursors, longer rows are
+    // bank-striped, see k_bank_stripe), so no binary search over rows.
     // Row descriptors: (first padded entry / 4) << 24 | true degree -- one 8-byte load per list.
     // Bits 52..62 hold (hub-bitmap slot + 1) of a node whose neighbour list is also kept as a
     // bitmap (0 = none); they are set only when every first-entry index fits 28 bits.
@@ -130,9 +130,9 @@ int build_hub_bitmaps(blp_graph* g, const int* u_deg_host, const int* b_deg_host
 // how many id-range passes side `n_side` needs on a device with `smem_optin` bytes per CTA
 void range_plan(int n_side, int smem_optin, int forced, int* n_ranges, int* range_words);
 constexpr int kMaxRanges = 255;
-// partition the middle rows of every ranged side by id range (reorder = false: rows already ascend)
-// and fill seg_off; `tmp` = scratch of max(u_adj_len, b_adj_len) ints when reordering
-int build_range_segments(blp_graph* g, bool reorder, int* tmp, cudaStream_t st);
+// partition the middle rows of every ranged side by id range and fill seg_off; `tmp` = device
+// scratch of max(u_adj_len, b_adj_len) ints
+int build_range_segments(blp_graph* g, int* tmp, cudaStream_t st);
 int init_device_state(blp_graph* g, int device, const blp_tuning& tune);
 void host_state_destroy(blp_graph* g);
 void weight_lut(int32_t max_deg, std::vector<unsigned>& lut);

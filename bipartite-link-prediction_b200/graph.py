@@ -87,9 +87,9 @@ class BipartiteGraph(object):
     def __init__(self, n_users, n_biz, edge_u, edge_b, device=None, user_ids=None, biz_ids=None,
                  build='device'):
         """build='device' (default): blp_graph_create_device -- CUDA int32 tensors are taken as they
-        are, anything else is uploaded first; radix sort and CSR build run on the GPU (6-11x faster
-        than the host builder on C2/C3);  build='host': blp_graph_create (C++ builder on the host
-        arrays).  Both yield the same scores."""
+        are, anything else is uploaded first; radix sort and CSR build run on the GPU;
+        build='host': host int32 arrays are handed to blp_graph_create, which uploads them and runs
+        the same build.  Both yield the same graph."""
         lib = _lib.load()
         if device is None:
             device = torch.cuda.current_device() if torch.cuda.is_available() else 0

@@ -105,7 +105,8 @@ int blp_device_count(int* count);
  * (similarity.py:16) and the node-id list of similarity.py:22,65: duplicate edges collapse, both
  * CSR directions, degree tables and the Adamic-Adar weight table 1/ln(deg) (similarity.py:121-123)
  * are made resident in HBM.  edge_u / edge_b are HOST arrays of n_edges local indices
- * (column 0 = user, column 1 = business of graph.txt, dataset_maker.py:197).
+ * (column 0 = user, column 1 = business of graph.txt, dataset_maker.py:197); they are copied to the
+ * device and built as blp_graph_create_device builds, on the legacy default stream.
  * Limits of the packed row descriptors: degrees below 2^24 and at most 2^30 adjacency entries per
  * direction after padding every row to a multiple of four (about a billion distinct edges);
  * beyond that the call fails with BLP_ERR_UNSUPPORTED.
@@ -117,8 +118,7 @@ int blp_graph_create(int32_t n_users, int32_t n_biz, int64_t n_edges,
  * The same, with the edge arrays already in DEVICE memory and the whole construction on the GPU:
  * 64-bit radix sort of the (user, business) keys, duplicate removal, both padded CSR directions,
  * bank striping of the rows, per-entry weights (SURVEY.md section 8f, the step in front of the
- * path).  Row order inside the CSR differs from the host builder's; every score is identical.
- * `stream` is a cudaStream_t; the call returns when the handle is ready.
+ * path).  `stream` is a cudaStream_t; the call returns when the handle is ready.
  */
 int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n_edges,
                             const int32_t* edge_u_dev, const int32_t* edge_b_dev,

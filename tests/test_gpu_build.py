@@ -1,4 +1,5 @@
-"""Graph construction on the device (blp_graph_create_device) against the host builder."""
+"""Graph construction on the device, reached through the host-array entry point (blp_graph_create)
+and the device-array one (blp_graph_create_device): against each other and against the C oracle."""
 import time
 
 import numpy as np
@@ -22,6 +23,8 @@ def same_graph(a, b):
 
 @pytest.mark.parametrize('name,n_pairs', [('C1', 40_000)])
 def test_device_build_scores_match_host_build(mods, name, n_pairs):
+    """Host arrays (blp_graph_create) and device arrays (blp_graph_create_device) of one edge list:
+    the same info, the same degrees and bit-identical scores."""
     graph, synth = mods
     cfg, eu, eb, pu, pv = synth.make_config(name, n_pairs=n_pairs)
     Gh = graph.BipartiteGraph(cfg['n_users'], cfg['n_biz'], eu, eb, build='host')
@@ -47,10 +50,12 @@ def test_device_build_small_and_odd_shapes(mods):
         got = G.score_pairs_host(pu, pv)
         want = c_oracle.score_pair_arrays(n_users, n_biz, eu, eb, pu, pv)
         check_against(got, want, pu.size)
-    for build in ('host', 'device'):
+    lib = pkg('_lib').load()
+    for build, api in (('host', b'blp_graph_create: '), ('device', b'blp_graph_create_device: ')):
         with pytest.raises(ValueError):
             graph.BipartiteGraph(4, 3, [0, 5], [0, 0], build=build)   # endpoint out of range
-    # the host builder on the same odd shapes
+        assert lib.blp_last_error().startswith(api + b'edge 1 '), lib.blp_last_error()
+    # the host-array entry point on the same odd shapes
     for n_users, n_biz, n_edges in ((1, 1, 1), (5, 3, 0), (3000, 2, 5000)):
         eu = rng.integers(0, n_users, n_edges)
         eb = rng.integers(0, n_biz, n_edges)

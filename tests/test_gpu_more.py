@@ -186,7 +186,7 @@ def test_id_range_passes_do_not_change_results(mods, monkeypatch):
     one = G.score_pairs_host(pu, pv, want_hop2=True)
     assert G.score_stats(lib.SIDE_USER)['range_passes'] == 1
     for r, build in (('2', 'device'), ('5', 'device'), ('3', 'host'), ('7', 'host')):
-        # a ranged side keeps its middle rows partitioned by range (both builders), and a pass
+        # a ranged side keeps its middle rows partitioned by range (either entry point), and a pass
         # walks only its segment of every list
         monkeypatch.setenv('BLP_RANGES', r)
         G2 = graph.BipartiteGraph(cfg['n_users'], cfg['n_biz'], eu, eb, build=build)
