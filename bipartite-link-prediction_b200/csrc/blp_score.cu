@@ -55,7 +55,7 @@ namespace blp {
 // ---------------------------------------------------------------------------------------------
 struct TileSmem {
     unsigned long long row[kTile];     // packed row descriptor of every list of the tile
-    unsigned long long aa[kTile];      // Q24.40 Adamic-Adar accumulators
+    unsigned long long aa[kTile];      // Adamic-Adar sums of Q1.31 weights (BLP_AA_FRAC_BITS)
     unsigned long long hub_bar;        // mbarrier the TMA bulk copy of a hub bitmap completes on
     int scan[kTile + 8];               // exclusive prefix of long-list chunk counts, [kTile] = total
     int coarse[32];                    // scan[8*i], contiguous: conflict-free first probe

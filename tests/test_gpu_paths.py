@@ -143,7 +143,9 @@ def test_light_group_corner_cases(mods, monkeypatch):
 
 def test_host_buffer_entry_point(mods):
     """blp_score_pairs_host (host buffers in and out, copies inside the call) == the device call,
-    for pinned session buffers, for plain pageable numpy arrays, and for every slice plan."""
+    for pinned session buffers and for plain pageable numpy arrays.  At 100,000 pairs every plan
+    collapses to one user slice and one business slice (slices are at least 65536 pairs); plans
+    with several slices are tested in test_gpu_entry_points.test_host_pipeline_slice_plan."""
     import ctypes
     graph, synth = mods
     lib_mod = pkg('_lib')
