@@ -13,12 +13,13 @@ CSRC = os.path.join(_HERE, 'csrc')
 INCLUDE = os.path.join(_ROOT, 'include')
 LIB_PATH = os.path.join(_HERE, 'libblp.so')
 SOURCES = ('blp_graph.cu', 'blp_build.cu', 'blp_score.cu', 'blp_host.cu', 'blp_hop3.cu', 'blp_eval.cu',
-           'blp_peer.cu')
+           'blp_peer.cu', 'blp_json.cu')
 
 BLP_OK = 0
 BLP_ERR_INVALID, BLP_ERR_CUDA, BLP_ERR_OOM, BLP_ERR_RANGE, BLP_ERR_UNSUPPORTED = -1, -2, -3, -4, -5
 SIDE_USER, SIDE_BUSINESS = 0, 1
 PATH_GROUPED, PATH_BIZ_INDEX = 0, 1     # blp_score_stats_t.path
+JSON_INT32, JSON_INT64, JSON_FLOAT64, JSON_FLOAT64_INT_ZERO = 0, 1, 2, 3   # blp_json_kind
 
 # every symbol include/blp.h declares
 EXPORTS = ('blp_version', 'blp_last_error', 'blp_device_count', 'blp_graph_create',
@@ -27,7 +28,8 @@ EXPORTS = ('blp_version', 'blp_last_error', 'blp_device_count', 'blp_graph_creat
            'blp_hop3_count', 'blp_hop3_fill', 'blp_eval_precision_at_k', 'blp_eval_roc_auc',
            'blp_score_pairs_host', 'blp_peer_alloc', 'blp_peer_open', 'blp_peer_close',
            'blp_peer_free', 'blp_derive_pairs', 'blp_peer_push', 'blp_edge_list_count',
-           'blp_edge_list_parse')
+           'blp_edge_list_parse', 'blp_examples_count', 'blp_examples_parse', 'blp_json_scores_count',
+           'blp_json_scores_fill')
 IPC_HANDLE_BYTES = 64
 
 
@@ -139,6 +141,16 @@ def load():
     lib.blp_edge_list_count.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p]
     lib.blp_edge_list_parse.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
                                         ctypes.c_void_p]
+    lib.blp_examples_count.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.POINTER(ctypes.c_int64),
+                                       ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p]
+    lib.blp_examples_parse.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64] + \
+        [ctypes.c_void_p] * 5
+    lib.blp_json_scores_count.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                          ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+                                          ctypes.c_void_p]
+    lib.blp_json_scores_fill.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+                                         ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p]
     lib.blp_peer_push.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
     lib.blp_derive_pairs.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64] + \
         [ctypes.c_void_p] * 8

@@ -374,6 +374,19 @@ int bits_for(unsigned v) {
 
 }  // namespace
 
+int exclusive_scan_u32(const unsigned* in, long long n, unsigned long long* out,
+                       unsigned long long* host_total, cudaStream_t st) {
+    if (n <= 0) {
+        if (host_total) *host_total = 0;
+        return BLP_OK;
+    }
+    Scanner scan;
+    scan.st = st;
+    const int rc = scan.run(in, n, false, out, host_total);
+    scan.release();
+    return rc;
+}
+
 // Sorts n 64-bit keys ascending on the bits named by `shifts` (8 bits from each shift, least
 // significant group first).  `keys` and `tmp` are device buffers of n entries; the sorted keys
 // end up where *sorted points (one of the two).  Stream-ordered, no host synchronisation.

@@ -138,6 +138,10 @@ void host_state_destroy(blp_graph* g);
 void weight_lut(int32_t max_deg, std::vector<unsigned>& lut);
 int radix_sort_u64(unsigned long long* keys, unsigned long long* tmp, long long n,
                    const std::vector<int>& shifts, cudaStream_t st, unsigned long long** sorted);
+// out[i] = in[0] + ... + in[i-1] for n 32-bit counts, stream-ordered; with host_total the grand
+// total is copied back (the stream is synchronised)
+int exclusive_scan_u32(const unsigned* in, long long n, unsigned long long* out,
+                       unsigned long long* host_total, cudaStream_t st);
 void set_error(const std::string& msg);
 int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
 blp_tuning read_tuning();

@@ -15,7 +15,10 @@ unchanged by eval.py:14-18, supervised_models.py:81-86 and supervised_classifier
 
 ``users`` / ``business`` flatten the examples into pair arrays and make ONE call per side into
 the CUDA library (``blp_score_pairs``), which yields all three methods at once; the per-method
-loop only selects which array is written where.  The three set-level helpers keep their
+loop only selects which array is written where.  ``main`` keeps the whole step on the device when
+``examples.json`` is in the device reader's grammar (what json.dumps writes for the reference's
+dict): the file is parsed there, scored, and every score file is formatted there, byte for byte
+what ``users`` / ``business`` write; any other file goes through ``json.load`` and those two.  The three set-level helpers keep their
 reference meaning on Python sets -- they are the public formulas, not the bulk path.
 """
 import math
@@ -29,6 +32,10 @@ from .graph import BipartiteGraph
 METHODS = ('common_neighbors', 'jaccard', 'adamic_adar', 'preferential_attachment')
 _COLUMN = {'common_neighbors': 'cn', 'jaccard': 'jaccard', 'adamic_adar': 'adamic',
            'preferential_attachment': 'pa'}
+# how _emit types each column in the file: cn / pa as ints, jaccard as floats, adamic as floats
+# except its untouched int 0
+_KIND = {'cn': _lib.JSON_INT32, 'pa': _lib.JSON_INT64, 'jaccard': _lib.JSON_FLOAT64,
+         'adamic': _lib.JSON_FLOAT64_INT_ZERO}
 
 PUNGraph = 'PUNGraph'   # placeholder for snap.PUNGraph in LoadEdgeList(PUNGraph, file, 0, 1)
 
@@ -40,12 +47,91 @@ def LoadEdgeList(graph_type, graph_file, src_col=0, dst_col=1, device=None):
 
 def main(example_file, graph_file, u_methods, u_outfiles, b_methods, b_outfiles, *,
          device=None, reproduce_reference_bug=False, sidecar=False):
-    examples = util.load_json(example_file)
+    ex = util.read_examples_device(example_file, device)
+    if ex is None:   # outside the device reader's grammar: json.load decides what the file means
+        examples = util.load_json(example_file)
+        G = LoadEdgeList(PUNGraph, graph_file, 0, 1, device=device)
+        users(examples, G, u_methods, u_outfiles, sidecar=sidecar)
+        business(examples, G, b_methods, b_outfiles, reproduce_reference_bug=reproduce_reference_bug,
+                 sidecar=sidecar)
+        return G
     G = LoadEdgeList(PUNGraph, graph_file, 0, 1, device=device)
-    users(examples, G, u_methods, u_outfiles, sidecar=sidecar)
-    business(examples, G, b_methods, b_outfiles, reproduce_reference_bug=reproduce_reference_bug,
-             sidecar=sidecar)
+    skip = ('adamic_adar',) if reproduce_reference_bug else ()
+    _main_device(G, ex, [(_lib.SIDE_USER, u_methods, u_outfiles, ()),
+                         (_lib.SIDE_BUSINESS, b_methods, b_outfiles, skip)], sidecar)
     return G
+
+
+def _lookup_device(table, ids):
+    """BipartiteGraph._lookup on the device: local index of every id, -1 where it is not in table."""
+    import torch
+    t = torch.from_numpy(table).to(ids.device)
+    pos = torch.searchsorted(t, ids).clamp_(max=t.numel() - 1)
+    return torch.where(t[pos] == ids, pos, -1).to(torch.int32)
+
+
+def _device_pairs(G, ex):
+    """Example arrays of read_examples_device -> (user_off, user_ids, biz_ids, per-pair user ids,
+    local user / business indices, in-graph mask), as _flatten + _score_side make them."""
+    import torch
+    dev = G.device
+    with torch.cuda.device(dev):
+        user_off, user_ids, biz_ids, _ = (t.to(dev) for t in ex)
+        ids_u = torch.repeat_interleave(user_ids, user_off[1:] - user_off[:-1],
+                                        output_size=biz_ids.numel())
+        lu, lb = _lookup_device(G.user_ids, ids_u), _lookup_device(G.biz_ids, biz_ids)
+        du = torch.from_numpy(G.degrees(_lib.SIDE_USER)).to(dev)
+        db = torch.from_numpy(G.degrees(_lib.SIDE_BUSINESS)).to(dev)
+        in_graph = ((lu >= 0) & (lb >= 0) & (du[lu.clamp(min=0).long()] > 0) &
+                    (db[lb.clamp(min=0).long()] > 0))
+    return user_off, user_ids, biz_ids, ids_u, lu, lb, in_graph
+
+
+def _write_side(pairs, res, methods, outfiles, skip=(), sidecar=False, buffers=None, stats=None):
+    """_emit's loop with the device formatter: one file per (method, file), from one side's
+    scores `res` (G.score_side's dict)."""
+    user_off, user_ids, biz_ids, ids_u, _, _, in_graph = pairs
+    for m, f in zip(methods, outfiles):
+        col = _COLUMN.get(m)
+        vals = None if col is None or m in skip else res[col]
+        util.write_scores_json_device(f, user_off, user_ids, biz_ids, in_graph, vals, _KIND.get(col),
+                                      buffers=buffers, stats=stats)
+        if sidecar:
+            _save_sidecar(f, *_sidecar_columns(ids_u, biz_ids, in_graph, vals, col))
+
+
+def _main_device(G, ex, sides, sidecar):
+    import torch
+    pairs = _device_pairs(G, ex)
+    _, _, _, _, lu, lb, _ = pairs
+    buffers = {}
+    with torch.cuda.device(G.device):
+        for side, methods, outfiles, skip in sides:
+            res = G.score_side(side, lu, lb, want_pa=True)
+            _write_side(pairs, res, methods, outfiles, skip, sidecar, buffers)
+
+
+def _sidecar_columns(ids_u, biz_ids, in_graph, vals, col):
+    """util.dict_to_columns of the dict _emit builds, computed from the pair arrays."""
+    import torch
+    if vals is None:                 # only the out-of-graph zeros
+        keep = ~in_graph
+        v = torch.zeros_like(ids_u, dtype=torch.float64)
+        im = torch.ones_like(in_graph)
+    else:
+        keep = torch.ones_like(in_graph)
+        v = torch.where(in_graph, vals.to(torch.float64), 0.0)
+        im = ~in_graph
+        if col in ('cn', 'pa'):
+            im = torch.ones_like(in_graph)
+        elif col == 'adamic':
+            im = im | (vals == 0)
+    return tuple(t[keep].cpu().numpy() for t in (ids_u, biz_ids, v, im))
+
+
+def _save_sidecar(f, u, b, v, im):
+    # columnar copy beside the JSON (SURVEY 8f rank 3); same content, no parsing
+    np.savez(f[:-5] + '.npz' if f.endswith('.json') else f + '.npz', u=u, b=b, v=v, int_mask=im)
 
 
 def _flatten(examples):
@@ -98,10 +184,8 @@ def _emit(examples, keys_u, keys_b, host, in_graph, methods, outfiles, skip_in_g
                 else:
                     sim[u][v] = int(vals[i])            # cn, pa, and adamic's untouched int 0
         util.write_json(sim, f)
-        if sidecar:   # columnar copy beside the JSON (SURVEY 8f rank 3); same content, no parsing
-            u, b, v, im = util.dict_to_columns(sim)
-            np.savez(f[:-5] + '.npz' if f.endswith('.json') else f + '.npz', u=u, b=b, v=v,
-                     int_mask=im)
+        if sidecar:
+            _save_sidecar(f, *util.dict_to_columns(sim))
         out.append(sim)
     return out
 

@@ -138,6 +138,61 @@ int blp_graph_create_device(int32_t n_users, int32_t n_biz, int64_t n_edges,
 int blp_edge_list_count(const char* text_dev, int64_t n_bytes, int64_t* n_lines_host, void* stream);
 int blp_edge_list_parse(const char* text_dev, int64_t n_bytes, int64_t n_lines, int64_t* col0_dev,
                         int64_t* col1_dev, void* stream);
+/*
+ * examples.json on the device: the reference's {"<user>": {"<business>": label}}
+ * (dataset_maker.py:142-159, read by similarity.py:14).  `text_dev` holds the file's bytes in
+ * DEVICE memory.  The grammar is exactly what json.dumps writes for such a dict, with any JSON
+ * whitespace (space, tab, CR, LF) between tokens: keys are canonical decimal integers ("0", or an
+ * optional '-' and [1-9][0-9]*, at most 18 digits, no escapes), labels are JSON integers that fit
+ * int32.  Anything else -- duplicate user keys or duplicate business keys of one user (json.load
+ * resolves those by "last wins, first position"), other key spellings, float / bool / null /
+ * string labels, deeper nesting, truncated or trailing text, a BOM, an empty file -- fails with
+ * BLP_ERR_UNSUPPORTED, and blp_last_error() names the byte offset: such files are for json.load.
+ *   blp_examples_count : *n_users_host / *n_pairs_host = users and (user, business) pairs
+ *   blp_examples_parse : DEVICE outputs in file order -- user_off (n_users + 1 int64: the pairs of
+ *                        user i are [user_off[i], user_off[i+1])), user_ids (n_users int64),
+ *                        biz_ids (n_pairs int64), labels (n_pairs int32, may be NULL)
+ * Both run on the caller's current device and return when done.
+ */
+int blp_examples_count(const char* text_dev, int64_t n_bytes, int64_t* n_users_host, int64_t* n_pairs_host,
+                       void* stream);
+int blp_examples_parse(const char* text_dev, int64_t n_bytes, int64_t n_users, int64_t n_pairs,
+                       int64_t* user_off_dev, int64_t* user_ids_dev, int64_t* biz_ids_dev, int32_t* labels_dev,
+                       void* stream);
+
+/* Value column of a score file (blp_json_scores_count / _fill), as similarity._emit types it. */
+typedef enum blp_json_kind {
+    BLP_JSON_INT32 = 0,            /* cn: int32, written as ints */
+    BLP_JSON_INT64 = 1,            /* pa: int64, written as ints */
+    BLP_JSON_FLOAT64 = 2,          /* jaccard: doubles, float.__repr__ */
+    BLP_JSON_FLOAT64_INT_ZERO = 3  /* adamic: doubles, but 0.0 written as the int 0 (similarity.py:116-126) */
+} blp_json_kind;
+
+/*
+ * Score file writer: the bytes util.write_json writes for the {"<u>": {"<b>": v}} dict of one
+ * method (similarity.py:49-61, 94-106), from DEVICE arrays.  The example users in file order are
+ * user_off (n_users + 1 int64, pairs of user i = [user_off[i], user_off[i+1])) and user_ids
+ * (int64); biz_ids (int64) and in_graph (one byte, 0 = an id of the pair is not in the graph) are
+ * per pair; `values` is the pair's column of type `kind`.  A pair not in the graph is written as
+ * the int 0 whatever the column; values == NULL writes only those zeros (an unknown method name,
+ * or in-graph entries the reference omits).  Keys are the decimal ids; floats are float.__repr__
+ * (Ryu shortest round trip), NaN / Infinity / -Infinity as json.dumps spells them.
+ * User i's text is  , "<u>": {"<b>": v, "<b>": v}  -- empty when none of its pairs is written --
+ * and the document is "{" + the concatenation of all users' texts without its first two bytes + "}"
+ * ("{}" when all are empty).
+ *   blp_json_scores_count : lengths_dev[i] (DEVICE, n_users int64) = bytes of user i's text
+ *   blp_json_scores_fill  : the texts of users [user_begin, user_end), user i's at
+ *                           out_dev + text_off_dev[i] - text_off_dev[user_begin], where text_off_dev
+ *                           is the caller's exclusive prefix sum of the lengths (DEVICE int64)
+ * so a large file is produced in chunks cut at user boundaries.  Both are asynchronous on `stream`.
+ */
+int blp_json_scores_count(const int64_t* user_off_dev, const int64_t* user_ids_dev, int64_t n_users,
+                          const int64_t* biz_ids_dev, const uint8_t* in_graph_dev, const void* values_dev,
+                          int kind, int64_t* lengths_dev, void* stream);
+int blp_json_scores_fill(const int64_t* user_off_dev, const int64_t* user_ids_dev, int64_t n_users,
+                         const int64_t* biz_ids_dev, const uint8_t* in_graph_dev, const void* values_dev,
+                         int kind, const int64_t* text_off_dev, int64_t user_begin, int64_t user_end,
+                         char* out_dev, void* stream);
 int blp_graph_destroy(blp_graph* g);
 int blp_graph_info(const blp_graph* g, blp_graph_info_t* info);
 
