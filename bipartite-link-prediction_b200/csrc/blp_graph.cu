@@ -5,7 +5,9 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstdio>
+#include <map>
 #include <mutex>
+#include <tuple>
 #include <vector>
 
 #include "blp_internal.h"
@@ -82,6 +84,36 @@ void release_scratch_pool(int device) {
         cudaMemPoolTrimTo(g_pool[device], 0);   // last handle gone: give the cached scratch back
         (void)cudaGetLastError();
     }
+}
+
+// The dynamic shared-memory opt-in is a property of (kernel, device) for the whole PROCESS, not of
+// a graph handle: handles of different size, possibly on different host threads, share it.  So it
+// is kept here, under one lock, and only ever raised: a small graph scored between two calls on a
+// large one cannot lower it under the large one's launch.  The occupancy of a (kernel, device,
+// block size, shared-memory size) does not change either, so it is queried once.
+namespace {
+std::mutex g_kernel_mutex;
+std::map<std::pair<const void*, int>, size_t> g_smem_optin;
+std::map<std::tuple<const void*, int, int, size_t>, int> g_ctas_per_sm;
+}  // namespace
+
+int kernel_ctas_per_sm(const void* kernel, int device, int threads, size_t smem, int* ctas_per_sm) {
+    std::lock_guard<std::mutex> lock(g_kernel_mutex);
+    size_t& granted = g_smem_optin[{kernel, device}];
+    if (smem > granted) {
+        BLP_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        granted = smem;
+    }
+    if (!ctas_per_sm) return BLP_OK;
+    const auto key = std::make_tuple(kernel, device, threads, smem);
+    auto it = g_ctas_per_sm.find(key);
+    if (it == g_ctas_per_sm.end()) {
+        int n = 0;
+        BLP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem));
+        it = g_ctas_per_sm.emplace(key, n).first;
+    }
+    *ctas_per_sm = it->second;
+    return BLP_OK;
 }
 
 // Device properties, tuning (read_tuning, called once by the builder), the scratch pool and the

@@ -189,18 +189,14 @@ int launch_hop3(blp_graph* g, Hop3Args a, bool fill, cudaStream_t st) {
         set_error("blp_hop3: the business bitmap alone exceeds one CTA's shared memory");
         return BLP_ERR_UNSUPPORTED;
     }
+    void (*const kernel)(Hop3Args) = fill ? k_hop3<true> : k_hop3<false>;
+    int per_sm = 0;
+    const int rc = kernel_ctas_per_sm((const void*)kernel, g->device, 256, smem, &per_sm);
+    if (rc != BLP_OK) return rc;
     int* counter = nullptr;
     BLP_CUDA_TRY(pool_alloc(g, (void**)&counter, sizeof(int), st));
     BLP_CUDA_TRY(cudaMemsetAsync(counter, 0, sizeof(int), st));
     a.work_counter = counter;
-    int per_sm = 0;
-    if (fill) {
-        BLP_CUDA_TRY(cudaFuncSetAttribute(k_hop3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        BLP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_hop3<true>, 256, smem));
-    } else {
-        BLP_CUDA_TRY(cudaFuncSetAttribute(k_hop3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        BLP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_hop3<false>, 256, smem));
-    }
     int grid = std::max(1, per_sm) * g->sm_count;
     if (global_users) {
         // at most 1 GiB of scratch bitmaps: fewer CTAs rather than more memory
@@ -209,8 +205,7 @@ int launch_hop3(blp_graph* g, Hop3Args a, bool fill, cudaStream_t st) {
         BLP_CUDA_TRY(pool_alloc(g, (void**)&a.ubm_global, per_cta * (size_t)grid, st));
         BLP_CUDA_TRY(cudaMemsetAsync(a.ubm_global, 0, per_cta * (size_t)grid, st));
     }
-    if (fill) k_hop3<true><<<grid, 256, smem, st>>>(a);
-    else k_hop3<false><<<grid, 256, smem, st>>>(a);
+    kernel<<<grid, 256, smem, st>>>(a);
     if (a.ubm_global) cudaFreeAsync(a.ubm_global, st);
     BLP_CUDA_TRY(cudaGetLastError());
     cudaFreeAsync(counter, st);

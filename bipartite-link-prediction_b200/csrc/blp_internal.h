@@ -47,9 +47,6 @@ struct blp_graph {
     // kept warm, trimmed when the last handle goes; see acquire_scratch_pool) -- the device's
     // default pool and other libraries' allocators are left alone
     cudaMemPool_t pool = nullptr;
-    // CTAs per SM of the scoring-kernel variants already configured: [nt 256/512/1024][ranged][rec]
-    int occ_cache[3][2][2] = {};
-    size_t occ_smem[3][2][2] = {};
     int32_t n_users = 0, n_biz = 0;
     int64_t n_edges_in = 0, n_edges = 0;
     int32_t n_users_in = 0, n_biz_in = 0, max_udeg = 0, max_bdeg = 0;
@@ -83,7 +80,6 @@ struct blp_graph {
     unsigned long long* xrow[2] = {nullptr, nullptr};   // expansion-side row descriptors (hubs tagged)
     unsigned* hub_bm[2] = {nullptr, nullptr};     // [n_hubs][bm_words]
     unsigned char* light[2] = {nullptr, nullptr}; // per grouping node of side s: 1 = warp-per-group kernel
-    int light_ctas_per_sm[2] = {};      // [rec]
     // |N(h) & N(y)| and its weight sum, OR-hub h (row) x bitmap node y (column), per side
     int* hubtab_cn[2] = {nullptr, nullptr};
     unsigned long long* hubtab_aa[2] = {nullptr, nullptr};
@@ -148,6 +144,11 @@ blp_tuning read_tuning();
 cudaMemPool_t acquire_scratch_pool(int device);
 void release_scratch_pool(int device);
 cudaError_t scratch_alloc(void** p, size_t bytes, cudaStream_t st);
+// Raises `kernel`'s dynamic shared-memory opt-in on `device` (the current device) to at least
+// `smem` -- never lowers it -- and, when ctas_per_sm != nullptr, returns how many CTAs of `threads`
+// threads with `smem` bytes fit on one SM.  Every kernel whose dynamic shared memory may exceed the
+// 48 KB default is configured here and nowhere else.
+int kernel_ctas_per_sm(const void* kernel, int device, int threads, size_t smem, int* ctas_per_sm);
 // stream-ordered scratch from the handle's own pool
 inline cudaError_t pool_alloc(blp_graph* g, void** p, size_t bytes, cudaStream_t st) {
     return g->pool ? cudaMallocFromPoolAsync(p, bytes, g->pool, st) : cudaMallocAsync(p, bytes, st);

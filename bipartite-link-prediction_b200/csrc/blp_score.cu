@@ -39,7 +39,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <mutex>
 #include <vector>
 
 #include "blp_internal.h"
@@ -710,37 +709,15 @@ __global__ void __launch_bounds__(NT, kThreadsPerSm / NT)
 }
 
 
-template <int NT, bool RANGED, bool REC>
-static int launch_side(const SideArgs& a, int grid, size_t smem, cudaStream_t st) {
-    // (the dynamic shared-memory opt-in covers this size: raise_smem_optin<>() ran just before)
-    k_score_side<NT, RANGED, REC><<<grid, NT, smem, st>>>(a);
-    BLP_CUDA_TRY(cudaGetLastError());
-    return BLP_OK;
-}
-
-// The dynamic shared-memory opt-in is a property of (kernel, device) for the whole PROCESS, not of
-// a graph handle: handles of different size share it.  It is kept in a process-wide table and only
-// ever raised, so a small graph scored between two calls on a large one cannot lower it.
-constexpr int kMaxDevices = 64;
-static std::mutex g_optin_mutex;
-template <int NT, bool RANGED, bool REC>
-static int raise_smem_optin(int device, size_t smem) {
-    static size_t granted[kMaxDevices] = {};
-    std::lock_guard<std::mutex> lock(g_optin_mutex);
-    if (device < 0 || device >= kMaxDevices || smem > granted[device]) {
-        BLP_CUDA_TRY(cudaFuncSetAttribute(k_score_side<NT, RANGED, REC>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        if (device >= 0 && device < kMaxDevices) granted[device] = smem;
-    }
-    return BLP_OK;
-}
-
-template <int NT, bool RANGED, bool REC>
-static int occupancy(size_t smem, int* ctas_per_sm) {
-    BLP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-        ctas_per_sm, k_score_side<NT, RANGED, REC>, NT, smem));
-    return BLP_OK;
-}
+// The variants of k_score_side, [block size 256 / 512 / 1024][ranged][rec]
+static void (*const kSideKernels[3][2][2])(SideArgs) = {
+    {{k_score_side<256, false, false>, k_score_side<256, false, true>},
+     {k_score_side<256, true, false>, k_score_side<256, true, true>}},
+    {{k_score_side<512, false, false>, k_score_side<512, false, true>},
+     {k_score_side<512, true, false>, k_score_side<512, true, true>}},
+    {{k_score_side<1024, false, false>, k_score_side<1024, false, true>},
+     {k_score_side<1024, true, false>, k_score_side<1024, true, true>}},
+};
 
 // The bitmap must hold bits 0..n_side (the last one is the padding sentinel).  When that does not
 // fit in one CTA's shared memory the id universe is cut into equal ranges and every group is
@@ -994,115 +971,100 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
 
     // ---- stream-ordered scratch + grouping
     const int n_keys = a.n_side + 1;
-    std::vector<void*> scratch;
-    // one stream-ordered block for all scratch of the call (an idle GPU would otherwise wait for
-    // a dozen allocator calls before the first kernel): carved by a bump pointer, 256-byte aligned
-    const size_t n_sz = (size_t)n, k_sz = (size_t)n_keys, i_sz = std::max(n_sz, k_sz);
-    const size_t arena_bytes = 4 * n_sz + 20 * i_sz + 8 * k_sz + 12 * n_sz + 24 * n_sz +
-                               (ranged ? 12 * n_sz : 0) + 8 * (k_sz / kScanTile + 1) + 64 * 256;
-    unsigned char* arena = nullptr;
-    size_t arena_used = 0;
-    {
-        cudaError_t e = pool_alloc(g, (void**)&arena, arena_bytes, st);
-        if (e != cudaSuccess) return blp::cuda_fail(e, "cudaMallocFromPoolAsync(scratch)", __FILE__, __LINE__);
-        scratch.push_back(arena);
-    }
-    auto alloc = [&](void** p, size_t bytes) -> cudaError_t {
-        const size_t at = (arena_used + 255) & ~(size_t)255;
-        if (at + bytes > arena_bytes) return cudaErrorMemoryAllocation;   // sizing bug, not OOM
-        *p = arena + at;
-        arena_used = at + bytes;
-        return cudaSuccess;
-    };
-    auto release = [&]() {
-        for (void* p : scratch) cudaFreeAsync(p, st);
-        scratch.clear();
-    };
-#define BLP_TRY_SCRATCH(expr)                                                    \
-    do {                                                                         \
-        cudaError_t e__ = (expr);                                                \
-        if (e__ != cudaSuccess) {                                                \
-            release();                                                           \
-            return blp::cuda_fail(e__, #expr, __FILE__, __LINE__);               \
-        }                                                                        \
-    } while (0)
-    int *keys = nullptr, *scalars = nullptr, *inv = nullptr;
-    int *item_key = nullptr, *item_start = nullptr, *item_end = nullptr;
-    BLP_TRY_SCRATCH(alloc((void**)&keys, sizeof(int) * (size_t)n));
-    // device-side scalars of the call, see the SC_* indices
-    BLP_TRY_SCRATCH(alloc((void**)&scalars, sizeof(int) * SC_COUNT));
-    BLP_TRY_SCRATCH(cudaMemsetAsync(scalars, 0, sizeof(int) * SC_COUNT, st));
-    if (ranged) {
-        BLP_TRY_SCRATCH(alloc((void**)&a.acc_cn, sizeof(int) * (size_t)n));
-        BLP_TRY_SCRATCH(alloc((void**)&a.acc_aa, sizeof(unsigned long long) * (size_t)n));
-    }
-
     // Pairs that already arrive grouped (the reference's examples.json stores them per user) need
     // no sort: the runs of equal keys are the work items when they average >= 4 pairs.  The
     // decision is taken on the device (k_decide_mode); the kernels of the mode not chosen exit at
     // once, so the call never waits for the host.
     const int force = us ? -1 : MODE_SORT;   // a per-user list is never grouped by business
-    unsigned* cnt = nullptr;
-    if (force == MODE_SORT) {   // the mode is certain: the keys pass counts the group sizes as well
-        BLP_TRY_SCRATCH(alloc((void**)&cnt, sizeof(unsigned) * (size_t)n_keys));
-        BLP_TRY_SCRATCH(cudaMemsetAsync(cnt, 0, sizeof(unsigned) * (size_t)n_keys, st));
+    const bool counted = force == MODE_SORT;  // mode certain: the keys pass counts the group sizes too
+    const size_t n_sz = (size_t)n, k_sz = (size_t)n_keys;
+    const size_t n_items_max = counted ? k_sz : std::max(k_sz, n_sz);
+    const int n_tiles = (n_keys + kScanTile - 1) / kScanTile;
+    // light / heavy split of the work items: light groups go to the warp-per-group kernel
+    const bool split = g->light[side] != nullptr;
+    int *keys = nullptr, *scalars = nullptr, *inv = nullptr, *tile_items = nullptr;
+    int *item_key = nullptr, *item_start = nullptr, *item_end = nullptr;
+    int *light_list = nullptr, *heavy_list = nullptr;
+    unsigned *cnt = nullptr, *grp_off = nullptr, *tile_sum = nullptr;
+    int2* pg = nullptr;
+    // One stream-ordered block holds all scratch of the call (an idle GPU would otherwise wait for
+    // a dozen allocator calls before the first kernel); every array starts 256-byte aligned.
+    const struct { void** p; size_t bytes; bool used; } layout[] = {
+        {(void**)&keys, sizeof(int) * n_sz, true},
+        {(void**)&scalars, sizeof(int) * SC_COUNT, true},   // device-side scalars, see SC_*
+        {(void**)&a.acc_cn, sizeof(int) * n_sz, ranged},    // carried between id-range passes
+        {(void**)&a.acc_aa, sizeof(unsigned long long) * n_sz, ranged},
+        {(void**)&cnt, sizeof(unsigned) * k_sz, true},
+        {(void**)&item_key, sizeof(int) * n_items_max, true},
+        {(void**)&item_start, sizeof(int) * n_items_max, true},
+        {(void**)&item_end, sizeof(int) * n_items_max, true},
+        {(void**)&inv, sizeof(int) * n_sz, true},
+        // grouped-order result records + gather pass: only when the sort mode is certain (the
+        // business side); a list whose mode is decided on the device writes its outputs directly
+        {(void**)&a.rec, sizeof(unsigned long long) * 3 * n_sz, counted},
+        {(void**)&grp_off, sizeof(unsigned) * k_sz, true},
+        {(void**)&pg, sizeof(int2) * n_sz, true},
+        {(void**)&tile_sum, sizeof(unsigned) * (size_t)n_tiles, true},
+        {(void**)&tile_items, sizeof(int) * (size_t)n_tiles, true},
+        {(void**)&light_list, sizeof(int) * n_items_max, split},
+        {(void**)&heavy_list, sizeof(int) * n_items_max, split},
+    };
+    auto align256 = [](size_t at) { return (at + 255) & ~(size_t)255; };
+    size_t block_bytes = 0;
+    for (const auto& s : layout)
+        if (s.used) block_bytes = align256(block_bytes) + s.bytes;
+    unsigned char* block = nullptr;
+    BLP_CUDA_TRY(pool_alloc(g, (void**)&block, block_bytes, st));
+    struct FreeOnReturn {   // stream-ordered: after every kernel this call queued on st
+        void* p;
+        cudaStream_t st;
+        ~FreeOnReturn() { cudaFreeAsync(p, st); }
+    } free_block{block, st};
+    size_t at = 0;
+    for (const auto& s : layout) {
+        if (!s.used) continue;
+        at = align256(at);
+        *s.p = block + at;
+        at += s.bytes;
     }
-    BLP_TRY_SCRATCH(cudaEventRecord(g->ev[side][0], st));
+
+    BLP_CUDA_TRY(cudaMemsetAsync(scalars, 0, sizeof(int) * SC_COUNT, st));
+    if (counted) BLP_CUDA_TRY(cudaMemsetAsync(cnt, 0, sizeof(unsigned) * k_sz, st));
+    BLP_CUDA_TRY(cudaEventRecord(g->ev[side][0], st));
     const int gblocks = (int)std::min<long long>((n + 255) / 256, (long long)g->sm_count * 16);
     int launches = 1;
-    k_group_keys<<<gblocks, 256, 0, st>>>(gx, gy, n, a.n_side, n_mid, g_deg, m_deg, keys, cnt);
-    BLP_TRY_SCRATCH(cudaGetLastError());
+    k_group_keys<<<gblocks, 256, 0, st>>>(gx, gy, n, a.n_side, n_mid, g_deg, m_deg, keys,
+                                          counted ? cnt : nullptr);
+    BLP_CUDA_TRY(cudaGetLastError());
 
     int* mode = scalars + 3;
-    if (force < 0) {
+    if (!counted) {
         k_count_runs<<<gblocks, 256, 0, st>>>(keys, n, (unsigned*)(scalars + 2));
-        BLP_TRY_SCRATCH(cudaGetLastError());
+        BLP_CUDA_TRY(cudaGetLastError());
         ++launches;
     }
     k_decide_mode<<<1, 1, 0, st>>>((const unsigned*)(scalars + 2), n, force, mode);
-    BLP_TRY_SCRATCH(cudaGetLastError());
+    BLP_CUDA_TRY(cudaGetLastError());
     ++launches;
-    const size_t n_items_max = force == MODE_SORT ? (size_t)n_keys : std::max((size_t)n_keys, (size_t)n);
-    BLP_TRY_SCRATCH(alloc((void**)&item_key, sizeof(int) * n_items_max));
-    BLP_TRY_SCRATCH(alloc((void**)&item_start, sizeof(int) * n_items_max));
-    BLP_TRY_SCRATCH(alloc((void**)&item_end, sizeof(int) * n_items_max));
-    if (force != MODE_SORT) {
+    if (!counted) {
         const int rblocks = (int)std::min<long long>((n + kRunCut - 1) / kRunCut,
                                                      (long long)g->sm_count * 8);
         k_runs_to_items<<<rblocks, 256, 0, st>>>(mode, keys, n, item_key, item_start, item_end,
                                                  scalars);
-        BLP_TRY_SCRATCH(cudaGetLastError());
+        BLP_CUDA_TRY(cudaGetLastError());
         ++launches;
-    }
-    unsigned* grp_off = nullptr;
-    int2* pg = nullptr;
-    const bool counted = cnt != nullptr;
-    BLP_TRY_SCRATCH(alloc((void**)&inv, sizeof(int) * (size_t)n));
-    // grouped-order result records + gather pass: only when the sort mode is certain (the
-    // business side); a list whose mode is decided on the device writes its outputs directly
-    if (force == MODE_SORT)
-        BLP_TRY_SCRATCH(alloc((void**)&a.rec, sizeof(unsigned long long) * 3 * (size_t)n));
-    if (!counted) BLP_TRY_SCRATCH(alloc((void**)&cnt, sizeof(unsigned) * (size_t)n_keys));
-    BLP_TRY_SCRATCH(alloc((void**)&grp_off, sizeof(unsigned) * (size_t)n_keys));
-    BLP_TRY_SCRATCH(alloc((void**)&pg, sizeof(int2) * (size_t)n));
-    if (!counted) {
-        BLP_TRY_SCRATCH(cudaMemsetAsync(cnt, 0, sizeof(unsigned) * (size_t)n_keys, st));
+        BLP_CUDA_TRY(cudaMemsetAsync(cnt, 0, sizeof(unsigned) * k_sz, st));
         k_group_count<<<gblocks, 256, 0, st>>>(mode, keys, n, cnt);
-        BLP_TRY_SCRATCH(cudaGetLastError());
+        BLP_CUDA_TRY(cudaGetLastError());
         ++launches;
     }
-    const int n_tiles = (n_keys + kScanTile - 1) / kScanTile;
-    unsigned* tile_sum = nullptr;
-    int* tile_items = nullptr;
-    BLP_TRY_SCRATCH(alloc((void**)&tile_sum, sizeof(unsigned) * (size_t)n_tiles));
-    BLP_TRY_SCRATCH(alloc((void**)&tile_items, sizeof(int) * (size_t)n_tiles));
     k_group_tile_sums<<<n_tiles, 1024, 0, st>>>(mode, cnt, n_keys, tile_sum, tile_items);
     k_group_tile_scan<<<1, 1024, 0, st>>>(mode, tile_sum, tile_items, n_tiles, scalars);
     k_group_tile_apply<<<n_tiles, 1024, 0, st>>>(mode, cnt, n_keys, tile_sum, tile_items, grp_off,
                                                   item_key, item_start, item_end);
-    BLP_TRY_SCRATCH(cudaGetLastError());
+    BLP_CUDA_TRY(cudaGetLastError());
     k_group_scatter<<<gblocks, 256, 0, st>>>(mode, keys, gy, n, grp_off, pg, inv);
-    BLP_TRY_SCRATCH(cudaGetLastError());
+    BLP_CUDA_TRY(cudaGetLastError());
     launches += 4;
     a.pg = pg;
     a.mode = mode;
@@ -1112,17 +1074,12 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
     a.item_end = item_end;
     a.n_items = scalars;
     a.work_counter = scalars + 1;
-    // light / heavy split of the work items: light groups go to the warp-per-group kernel
-    const bool split = g->light[side] != nullptr;
     SideArgs la{};
     if (split) {
-        int *light_list = nullptr, *heavy_list = nullptr;
-        BLP_TRY_SCRATCH(alloc((void**)&light_list, sizeof(int) * n_items_max));
-        BLP_TRY_SCRATCH(alloc((void**)&heavy_list, sizeof(int) * n_items_max));
         const int sblocks = (int)std::min<size_t>((n_items_max + 255) / 256, (size_t)g->sm_count * 8);
         k_split_items<<<sblocks, 256, 0, st>>>(scalars, item_key, g->light[side], a.n_side,
                                                light_list, heavy_list);
-        BLP_TRY_SCRATCH(cudaGetLastError());
+        BLP_CUDA_TRY(cudaGetLastError());
         ++launches;
         la = a;
         la.item_list = light_list;
@@ -1131,59 +1088,31 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
         a.item_list = heavy_list;
         a.n_items = scalars + SC_N_HEAVY;
     }
-    BLP_TRY_SCRATCH(cudaEventRecord(g->ev[side][1], st));
+    BLP_CUDA_TRY(cudaEventRecord(g->ev[side][1], st));
 
     // ---- persistent scoring grid: as many CTAs per SM as the bitmap allows
-    int per_sm = 0, nt = 0, rc = BLP_OK;
     const size_t budget = (size_t)g->max_smem_optin;
-    if (smem * 4 + 4096 <= budget) nt = 256;
-    else if (smem * 2 + 2048 <= budget) nt = 512;
-    else nt = 1024;
+    const int nt = smem * 4 + 4096 <= budget ? 256 : (smem * 2 + 2048 <= budget ? 512 : 1024);
     const int use_sms = std::max(1, g->sm_count - g->reserve_sms);
     const bool rec_mode = a.rec != nullptr;
-    // the occupancy query and the shared-memory opt-in are done once per variant and size
-    const int nt_i = nt == 256 ? 0 : (nt == 512 ? 1 : 2);
-    int& occ_slot = g->occ_cache[nt_i][ranged ? 1 : 0][rec_mode ? 1 : 0];
-    size_t& occ_smem = g->occ_smem[nt_i][ranged ? 1 : 0][rec_mode ? 1 : 0];
-#define BLP_DISPATCH(NTV, RV)                                               \
-    do {                                                                    \
-        rc = rec_mode ? raise_smem_optin<NTV, RV, true>(g->device, smem)    \
-                      : raise_smem_optin<NTV, RV, false>(g->device, smem);  \
-        if (rc != BLP_OK) break;                                            \
-        if (occ_slot > 0 && occ_smem == smem) {                             \
-            per_sm = occ_slot;                                              \
-        } else {                                                            \
-            rc = rec_mode ? occupancy<NTV, RV, true>(smem, &per_sm)         \
-                          : occupancy<NTV, RV, false>(smem, &per_sm);       \
-            if (rc == BLP_OK) {                                             \
-                occ_slot = per_sm;                                          \
-                occ_smem = smem;                                            \
-            }                                                               \
-        }                                                                   \
-        if (rc == BLP_OK && per_sm < 1) {                                   \
-            set_error("blp_score_pairs: scoring kernel does not fit on an SM"); \
-            rc = BLP_ERR_UNSUPPORTED;                                       \
-        }                                                                   \
-        if (rc == BLP_OK)                                                   \
-            rc = rec_mode ? launch_side<NTV, RV, true>(a, per_sm * use_sms, smem, st)  \
-                          : launch_side<NTV, RV, false>(a, per_sm * use_sms, smem, st); \
-    } while (0)
+    void (*const kernel)(SideArgs) = kSideKernels[nt == 256 ? 0 : (nt == 512 ? 1 : 2)][ranged][rec_mode];
     // The CTA kernel goes first and the warp-per-group kernel beside it on the handle's side
     // stream: both are persistent work-queue grids, so as the CTA kernel's blocks retire (its
     // groups are few and large, the tail is long) the small warp-per-group blocks fill the SMs.
     if (split) {
-        BLP_TRY_SCRATCH(cudaEventRecord(g->ev_fork[side], st));
-        BLP_TRY_SCRATCH(cudaStreamWaitEvent(g->side_stream, g->ev_fork[side], 0));
+        BLP_CUDA_TRY(cudaEventRecord(g->ev_fork[side], st));
+        BLP_CUDA_TRY(cudaStreamWaitEvent(g->side_stream, g->ev_fork[side], 0));
     }
-    if (nt == 256) {
-        if (ranged) BLP_DISPATCH(256, true); else BLP_DISPATCH(256, false);
-    } else if (nt == 512) {
-        if (ranged) BLP_DISPATCH(512, true); else BLP_DISPATCH(512, false);
-    } else {
-        if (ranged) BLP_DISPATCH(1024, true); else BLP_DISPATCH(1024, false);
+    int per_sm = 0;
+    int rc = kernel_ctas_per_sm((const void*)kernel, g->device, nt, smem, &per_sm);
+    if (rc != BLP_OK) return rc;
+    if (per_sm < 1) {
+        set_error("blp_score_pairs: scoring kernel does not fit on an SM");
+        return BLP_ERR_UNSUPPORTED;
     }
-#undef BLP_DISPATCH
-    if (rc == BLP_OK && split) {
+    kernel<<<per_sm * use_sms, nt, smem, st>>>(a);
+    BLP_CUDA_TRY(cudaGetLastError());
+    if (split) {
         cudaStream_t lst = g->side_stream;
         rc = rec_mode ? launch_light<kLightCap, kLightSlots, kLightWarps, true>(g, la, use_sms, lst)
                       : launch_light<kLightCap, kLightSlots, kLightWarps, false>(g, la, use_sms, lst);
@@ -1194,27 +1123,26 @@ extern "C" int blp_score_pairs(blp_graph* g, int side, const int32_t* pair_u, co
             if (cudaStreamWaitEvent(st, g->ev[side][3], 0) != cudaSuccess)
                 rc = blp::cuda_fail(cudaGetLastError(), "joining the side stream", __FILE__, __LINE__);
         }
-        if (rc != BLP_OK) cudaStreamSynchronize(lst);   // scratch is freed below
+        if (rc != BLP_OK) {
+            cudaStreamSynchronize(lst);   // before the scratch block is freed on st
+            return rc;
+        }
     }
-    if (rc == BLP_OK && a.rec) {
+    if (a.rec) {
         k_unpermute<<<gblocks, 256, 0, st>>>(a.mode, a.rec, inv, n, a.cn, a.uni, a.jac, a.aa);
-        if (cudaGetLastError() != cudaSuccess) rc = BLP_ERR_CUDA;
+        BLP_CUDA_TRY(cudaGetLastError());
         ++launches;
     }
-    if (rc == BLP_OK) {
-        // work-item counts of this call, for blp_score_stats (the scalars live in scratch)
-        cudaMemcpyAsync(g->d_counts[side], scalars + SC_N_ITEMS, sizeof(int), cudaMemcpyDeviceToDevice, st);
-        cudaMemcpyAsync(g->d_counts[side] + 1, scalars + SC_N_LIGHT, sizeof(int), cudaMemcpyDeviceToDevice, st);
-        if (cudaEventRecord(g->ev[side][2], st) == cudaSuccess) g->ev_recorded[side] = true;
-        stats.ctas = per_sm * use_sms;
-        stats.threads_per_cta = nt;
-        stats.smem_bytes = (int)smem;
-        stats.kernel_launches = launches + 1;
-        stats.range_passes = n_ranges;
-    }
-    release();
-#undef BLP_TRY_SCRATCH
-    return rc;
+    // work-item counts of this call, for blp_score_stats (the scalars live in scratch)
+    cudaMemcpyAsync(g->d_counts[side], scalars + SC_N_ITEMS, sizeof(int), cudaMemcpyDeviceToDevice, st);
+    cudaMemcpyAsync(g->d_counts[side] + 1, scalars + SC_N_LIGHT, sizeof(int), cudaMemcpyDeviceToDevice, st);
+    if (cudaEventRecord(g->ev[side][2], st) == cudaSuccess) g->ev_recorded[side] = true;
+    stats.ctas = per_sm * use_sms;
+    stats.threads_per_cta = nt;
+    stats.smem_bytes = (int)smem;
+    stats.kernel_launches = launches + 1;
+    stats.range_passes = n_ranges;
+    return BLP_OK;
 }
 
 #ifdef BLP_PHASE_TIMING

@@ -212,12 +212,12 @@ int build_biz_index(blp_graph* g, const int* b_deg_host) {
     for (int b = 0; b < n_biz; ++b) order[b] = b;
     std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return b_deg_host[x] > b_deg_host[y]; });
     for (int r = 0; r < n_biz; ++r) rank[order[r]] = r;
+    const size_t smem = (size_t)words * 4;
+    const int rc = kernel_ctas_per_sm((const void*)k_build_biz_index, g->device, kIndexBuildThreads, smem, nullptr);
+    if (rc != BLP_OK) return rc;
     int* d_rank = nullptr;
     BLP_CUDA_TRY(cudaMalloc((void**)&d_rank, sizeof(int) * (size_t)n_biz));
     cudaError_t e = cudaMemcpy(d_rank, rank.data(), sizeof(int) * (size_t)n_biz, cudaMemcpyHostToDevice);
-    const size_t smem = (size_t)words * 4;
-    if (e == cudaSuccess && smem > 48 * 1024)
-        e = cudaFuncSetAttribute(k_build_biz_index, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e == cudaSuccess) {
         k_rank_ids<<<g->sm_count * 8, 256>>>(g->u_adj, g->u_adj_len, d_rank, n_biz, g->biz_radj);
         k_build_biz_index<<<std::min(n_biz, g->sm_count * 8), kIndexBuildThreads, smem>>>(

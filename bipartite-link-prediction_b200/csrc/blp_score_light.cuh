@@ -495,18 +495,13 @@ __global__ void k_hub_tables(const int* __restrict__ or_nodes, int n_bm,
 template <int CAP, int SLOTS, int WARPS, bool REC>
 static int launch_light(blp_graph* g, const SideArgs& a, int use_sms, cudaStream_t st) {
     const size_t smem = sizeof(LightSmem<CAP, SLOTS>) * WARPS;
-    int& per_sm = g->light_ctas_per_sm[REC ? 1 : 0];
-    if (per_sm == 0) {
-        BLP_CUDA_TRY(cudaFuncSetAttribute(k_score_light<CAP, SLOTS, WARPS, REC>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int occ = 0;
-        BLP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-            &occ, k_score_light<CAP, SLOTS, WARPS, REC>, WARPS * 32, smem));
-        if (occ < 1) {
-            set_error("blp_score_pairs: the warp-per-group kernel does not fit on an SM");
-            return BLP_ERR_UNSUPPORTED;
-        }
-        per_sm = occ;
+    int per_sm = 0;
+    const int rc = kernel_ctas_per_sm((const void*)k_score_light<CAP, SLOTS, WARPS, REC>, g->device,
+                                      WARPS * 32, smem, &per_sm);
+    if (rc != BLP_OK) return rc;
+    if (per_sm < 1) {
+        set_error("blp_score_pairs: the warp-per-group kernel does not fit on an SM");
+        return BLP_ERR_UNSUPPORTED;
     }
     k_score_light<CAP, SLOTS, WARPS, REC><<<per_sm * use_sms, WARPS * 32, smem, st>>>(a);
     BLP_CUDA_TRY(cudaGetLastError());
