@@ -209,6 +209,7 @@ extern "C" int blp_graph_destroy(blp_graph* g) {
     cudaFree(g->biz_index);
     cudaFree(g->biz_hop2);
     cudaFree(g->biz_radj);
+    cudaFree(g->biz_rank);
     for (int sd = 0; sd < 2; ++sd)
         for (int k = 0; k < 4; ++k)
             if (g->ev[sd][k]) cudaEventDestroy(g->ev[sd][k]);

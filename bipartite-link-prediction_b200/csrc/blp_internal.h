@@ -98,15 +98,18 @@ struct blp_graph {
     int probe_ratio = 2;                              // probe when deg(y) >= ratio * |hop2(x)|
     bool row_slots[2] = {false, false};               // slot bits present in the middle rows of side s
     // Business index: the business x business co-review relation as one bitmap row per business,
-    // row b = hop2(b) (businesses sharing a reviewer with b, b itself excluded), biz_index_words
-    // words each, and |hop2(b)| per business.  Built once per graph when the business side runs
-    // unranged and the rows fit the cap (build_biz_index); the business side then scores every
-    // pair by testing N(u) against row b, with no grouping.  nullptr = the grouped path.
-    // Its columns are business RANKS by degree (blp_score_index.cuh); biz_radj = u_adj with every
+    // biz_index_words words each, and |hop2(b)| per business (biz_hop2, by id).  Rows AND columns
+    // are business RANKS by degree (biz_rank[b], rank 0 = the most-reviewed business): row rank(b)
+    // holds hop2(b) (businesses sharing a reviewer with b, b itself excluded).  The relation is
+    // symmetric, so the kernel reads the bit of (b, b') at row max(rank b, rank b'), column min
+    // (blp_score_index.cuh).  Built once per graph when the business side runs unranged and the
+    // rows fit the cap (build_biz_index); the business side then scores every pair by testing N(u)
+    // against it, with no grouping.  nullptr = the grouped path.  biz_radj = u_adj with every
     // business id replaced by its rank.
     unsigned* biz_index = nullptr;
     int* biz_hop2 = nullptr;
     int* biz_radj = nullptr;
+    int* biz_rank = nullptr;
     int biz_index_words = 0;
     int64_t biz_index_bytes = 0;
     float biz_index_build_ms = 0.f;

@@ -22,8 +22,8 @@
 // warp pass each (degree-bucketed scheduling without separate launches).  The business side of a
 // handle WITH an index (hop2(b) of every business precomputed once per graph as a bitmap row:
 // C1-C4) is one pass over the pairs in the caller's order, k_score_biz_indexed: a lane tests N(u)
-// against row b, the warp walks the rare long N(u) together -- no grouping, no expansion, no
-// un-permute.  Both paths end in the same epilogue (emit_pair).
+// against b's bits, the CTA walks the rare long N(u) of its pairs together -- no grouping, no
+// expansion, no un-permute.  Both paths end in the same epilogue (emit_pair).
 //
 // Layout of the translation unit:
 //   blp_score_common.cuh  launch arguments (SideArgs), row-descriptor accessors, streaming loads,

@@ -4,7 +4,7 @@
 // b' is in hop2(b) iff b' != b and b, b' share a reviewer -- a relation of the graph alone, the
 // same on every call.  So it is built once per graph as one bitmap row per business (the
 // co-review pattern of A^T A without its diagonal), and a call scores every pair in the caller's
-// order by testing N(u) (4.8 ids on average on C2) against row b: no counting sort, no per-call
+// order by testing N(u) (4.8 ids on average on C2) against b's bits: no counting sort, no per-call
 // expansion of hop2(b), no grouped-order records and no un-permute pass.  The index lives beside the
 // graph for the handle's lifetime; it is read-only after the build.  The rows take
 // n_biz^2 / 8 bytes (C2: 465 MB, C3 / C4: 4.5 GB), so a graph with too many businesses (C5) and a
@@ -22,15 +22,18 @@
 namespace blp {
 
 constexpr int kIndexBuildThreads = 512;
-constexpr int kIndexScoreThreads = 256;
+constexpr int kIndexScoreThreads = 256;   // a power of two (the long-list word search halves it)
 // pairs with deg(u) <= this are scored by their own lane (C2: 96.6 % of the pairs); the longer
-// ones by the whole warp, 128 ids per pass
+// lists by the whole CTA
 constexpr int kIndexLaneDeg = 16;
 
-// Columns are kept in DEGREE-RANK order: bit rank(b') of a row stands for business b' (rank 0 =
-// the most-reviewed business).  The ids a pair tests are the businesses of N(u), and reviews are
-// power-law distributed over businesses, so most tests land in the first few hundred bits of a
-// row: a few 32-byte sectors per row instead of one per id.  The rows themselves stay in id order.
+// Rows and columns are kept in DEGREE-RANK order (rank 0 = the most-reviewed business): row
+// rank(b) holds hop2(b), bit rank(b') of it stands for business b'.  The relation is symmetric and
+// its diagonal is clear, so the bit of (b, b') is read at row max(rank b, rank b'), column min.
+// The ids a pair tests are the businesses of N(u), and reviews are power-law distributed over
+// businesses, so the tests gather in the low-rank columns: on C2 the 48 M tests of one call touch
+// 5.8 M distinct 32-byte sectors (8.6 M when row b is read at column rank(b')), and the hottest
+// 96 MiB of them answer 92 % of the tests (tools/biz_sectors.py).
 // u_radj is u_adj with every business id replaced by its rank (padding stays the sentinel n_biz,
 // whose bit is never set); the weights u_adjw stay parallel to it.
 __global__ void k_rank_ids(const int* __restrict__ ids, long long n, const int* __restrict__ rank,
@@ -44,7 +47,7 @@ __global__ void k_rank_ids(const int* __restrict__ ids, long long n, const int* 
 
 // One CTA per business (grid-stride): hop2(b) = U_{u in N(b)} N(u) \ {b} in a shared-memory bitmap
 // over ranks.  Warps take the users of N(b) round-robin and walk their (ranked) lists id by id; the
-// row is then written with 128-bit stores and its popcount is |hop2(b)|.  (The hub bitmaps of the
+// bitmap is then written to row rank(b) with 128-bit stores and its popcount is |hop2(b)|.  (The hub bitmaps of the
 // business side are over ids, not ranks, so they are not used here: the whole build walks
 // sum_u deg(u)^2 ids once per graph -- 205 M on C2.)
 __global__ void __launch_bounds__(kIndexBuildThreads) k_build_biz_index(
@@ -80,7 +83,7 @@ __global__ void __launch_bounds__(kIndexBuildThreads) k_build_biz_index(
             bm[r >> 5] &= ~(1u << (r & 31));
         }
         __syncthreads();
-        uint4* dst = reinterpret_cast<uint4*>(index + (size_t)b * words);
+        uint4* dst = reinterpret_cast<uint4*>(index + (size_t)rank[b] * words);
         int cnt = 0;
         for (int i = tid; i < n4; i += kIndexBuildThreads) {
             const uint4 v = bm4[i];
@@ -95,26 +98,49 @@ __global__ void __launch_bounds__(kIndexBuildThreads) k_build_biz_index(
     }
 }
 
-// four ids of N(u) (padding: the sentinel n_biz, whose bit is never set, weight 0) against row b
-__device__ __forceinline__ void index_test4(const unsigned* row, int4 v, uint4 wt, unsigned& cnt,
-                                            unsigned long long& acc, unsigned long long pol) {
-    const unsigned w0 = ldg_keep(row + (v.x >> 5), pol), w1 = ldg_keep(row + (v.y >> 5), pol);
-    const unsigned w2 = ldg_keep(row + (v.z >> 5), pol), w3 = ldg_keep(row + (v.w >> 5), pol);
-    const unsigned h0 = (w0 >> (v.x & 31)) & 1u, h1 = (w1 >> (v.y & 31)) & 1u;
-    const unsigned h2 = (w2 >> (v.z & 31)) & 1u, h3 = (w3 >> (v.w & 31)) & 1u;
+// Bit (rb, r) of the index: row max, column min.  Padding (r = the sentinel n_biz, weight 0) stays
+// on the pair's own row rb at column n_biz, whose bit is never set: row n_biz does not exist.
+__device__ __forceinline__ unsigned index_bit(const unsigned* index, int words, int n_biz, int rb, int r,
+                                              unsigned long long pol) {
+    const bool swap = r > rb && r < n_biz;
+    const int row = swap ? r : rb, col = swap ? rb : r;
+    return (ldg_keep(index + (size_t)row * (size_t)words + (col >> 5), pol) >> (col & 31)) & 1u;
+}
+
+// four ids of N(u) (as ranks) against business rank rb
+__device__ __forceinline__ void index_test4(const unsigned* index, int words, int n_biz, int rb, int4 v,
+                                            uint4 wt, unsigned& cnt, unsigned long long& acc,
+                                            unsigned long long pol) {
+    const unsigned h0 = index_bit(index, words, n_biz, rb, v.x, pol);
+    const unsigned h1 = index_bit(index, words, n_biz, rb, v.y, pol);
+    const unsigned h2 = index_bit(index, words, n_biz, rb, v.z, pol);
+    const unsigned h3 = index_bit(index, words, n_biz, rb, v.w, pol);
     cnt += h0 + h1 + h2 + h3;
     acc += (unsigned long long)(h0 * wt.x) + (unsigned long long)(h1 * wt.y) +
            (unsigned long long)(h2 * wt.z) + (unsigned long long)(h3 * wt.w);
 }
 
 // One thread per pair, in the caller's order (x = business b, y = user u).  A lane scores its own
-// pair when deg(u) <= kIndexLaneDeg; the warp then walks the longer lists of its 32 pairs together.
+// pair when deg(u) <= kIndexLaneDeg.  The longer lists of the CTA's pairs are cut into their 128-bit
+// words, laid end to end, and all threads of the CTA take those words round-robin, adding their hits
+// to the pair's counters in shared memory (integer sums: the order does not matter).  Pairs come in
+// runs of one user, so a user with thousands of businesses fills a whole warp with long lists: on
+// one warp its run takes sum(deg) / 128 dependent load rounds (C2: up to 714), spread over the CTA
+// an eighth of that.
 __global__ void __launch_bounds__(kIndexScoreThreads) k_score_biz_indexed(
     SideArgs a, const int* __restrict__ pair_b, const int* __restrict__ pair_u, long long n, int n_mid,
     const int* __restrict__ b_deg, const int* __restrict__ u_deg, const int* __restrict__ u_radj,
-    const unsigned* __restrict__ index, const int* __restrict__ hop2v, int words) {
-    const long long i = (long long)blockIdx.x * kIndexScoreThreads + threadIdx.x;
-    const int lane = threadIdx.x & 31;
+    const unsigned* __restrict__ index, const int* __restrict__ hop2v, const int* __restrict__ rank,
+    int words) {
+    constexpr int NW = kIndexScoreThreads / 32;
+    __shared__ int s_warp[NW];
+    __shared__ int s_end[kIndexScoreThreads];   // end of each pair's long-list words (inclusive scan)
+    __shared__ unsigned long long s_row[kIndexScoreThreads];
+    __shared__ int s_rb[kIndexScoreThreads];
+    __shared__ unsigned s_cnt[kIndexScoreThreads];
+    __shared__ unsigned long long s_acc[kIndexScoreThreads];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const long long i = (long long)blockIdx.x * kIndexScoreThreads + tid;
     const unsigned long long pol = l2_keep_policy();
     const int4* adj4 = reinterpret_cast<const int4*>(u_radj);   // N(u) as ranks, beside u_adjw
     const uint4* adjw4 = reinterpret_cast<const uint4*>(a.m_adjw);
@@ -126,41 +152,76 @@ __global__ void __launch_bounds__(kIndexScoreThreads) k_score_biz_indexed(
     }
     const bool valid = in && group_key(b, u, a.n_side, n_mid, b_deg, u_deg) < a.n_side;
     unsigned long long urow = 0ull;
-    int hop2 = 0;
+    int hop2 = 0, rb = 0;
     if (valid) {
         urow = a.m_row[u];
         hop2 = hop2v[b];
+        rb = rank[b];
     }
-    const int pdeg = row_deg(urow);
-    const unsigned* row = index + (size_t)(valid ? b : 0) * (size_t)words;
+    const int pdeg = row_deg(urow);   // 0 for an invalid pair: nothing to walk
+    const int n_biz = a.n_side;
+    const int n4 = (pdeg + 3) >> 2;
+    const bool lng = pdeg > kIndexLaneDeg;
+    int end = lng ? n4 : 0;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int t = __shfl_up_sync(kFull, end, d);
+        if (lane >= d) end += t;
+    }
+    if (lane == 31) s_warp[warp] = end;
+    s_row[tid] = urow;
+    s_rb[tid] = rb;
+    s_cnt[tid] = 0u;
+    s_acc[tid] = 0ull;
+    __syncthreads();
+    int total = 0;
+#pragma unroll
+    for (int w = 0; w < NW; ++w) {
+        if (w == warp) end += total;
+        total += s_warp[w];
+    }
+    s_end[tid] = end;
+
     unsigned cnt = 0;
     unsigned long long acc = 0ull;
-    const bool own = valid && pdeg <= kIndexLaneDeg;
-    if (own) {
+    if (!lng) {
         const long long f4 = row_first4(urow);
-        const int n4 = (pdeg + 3) >> 2;
         for (int k = 0; k < n4; ++k)
-            index_test4(row, ldg_stream(adj4 + f4 + k, pol), ldg_stream_u(adjw4 + f4 + k, pol), cnt, acc,
-                        pol);
+            index_test4(index, words, n_biz, rb, ldg_stream(adj4 + f4 + k, pol), ldg_stream_u(adjw4 + f4 + k, pol),
+                        cnt, acc, pol);
     }
-    unsigned todo = __ballot_sync(kFull, valid && !own);
-    while (todo) {
-        const int src = __ffs(todo) - 1;
-        todo &= todo - 1;
-        const unsigned long long r = __shfl_sync(kFull, urow, src);
-        const unsigned* rb = index + (size_t)__shfl_sync(kFull, b, src) * (size_t)words;
-        const long long f4 = row_first4(r);
-        const int n4 = (row_deg(r) + 3) >> 2;
+    if (total > 0) {   // the same on every thread of the CTA
+        __syncthreads();
+        int cur = -1;
         unsigned c = 0;
         unsigned long long s = 0ull;
-        for (int k = lane; k < n4; k += 32)
-            index_test4(rb, ldg_stream(adj4 + f4 + k, pol), ldg_stream_u(adjw4 + f4 + k, pol), c, s, pol);
-        c = __reduce_add_sync(kFull, c);
+        for (int j = tid; j < total; j += kIndexScoreThreads) {
+            int p = 0;   // the pair word j belongs to: the first with s_end[p] > j
 #pragma unroll
-        for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(kFull, s, d);
-        if (lane == src) {
-            cnt = c;
-            acc = s;
+            for (int step = kIndexScoreThreads / 2; step > 0; step >>= 1)
+                if (s_end[p + step - 1] <= j) p += step;
+            if (p != cur) {
+                if (cur >= 0) {
+                    atomicAdd(&s_cnt[cur], c);
+                    atomicAdd(&s_acc[cur], s);
+                }
+                cur = p;
+                c = 0;
+                s = 0ull;
+            }
+            const unsigned long long r = s_row[p];
+            const long long w4 = row_first4(r) + j - (s_end[p] - ((row_deg(r) + 3) >> 2));
+            index_test4(index, words, n_biz, s_rb[p], ldg_stream(adj4 + w4, pol), ldg_stream_u(adjw4 + w4, pol),
+                        c, s, pol);
+        }
+        if (cur >= 0) {
+            atomicAdd(&s_cnt[cur], c);
+            atomicAdd(&s_acc[cur], s);
+        }
+        __syncthreads();
+        if (lng) {
+            cnt = s_cnt[tid];
+            acc = s_acc[tid];
         }
     }
     if (in) emit_pair<false>(a, i, (int)i, valid, (int)cnt, hop2, (valid && a.pa) ? b_deg[b] : 0, pdeg, acc);
@@ -188,22 +249,24 @@ void reserve_biz_index(blp_graph* g) {
     if (mode < 0 && (bytes > cap || bytes > free_b / 2)) return;
     if (cudaMalloc((void**)&g->biz_index, bytes) != cudaSuccess ||
         cudaMalloc((void**)&g->biz_hop2, sizeof(int) * (size_t)g->n_biz) != cudaSuccess ||
-        cudaMalloc((void**)&g->biz_radj, sizeof(int) * (size_t)g->u_adj_len) != cudaSuccess) {
+        cudaMalloc((void**)&g->biz_radj, sizeof(int) * (size_t)g->u_adj_len) != cudaSuccess ||
+        cudaMalloc((void**)&g->biz_rank, sizeof(int) * (size_t)g->n_biz) != cudaSuccess) {
         (void)cudaGetLastError();
         cudaFree(g->biz_index);
         cudaFree(g->biz_hop2);
         cudaFree(g->biz_radj);
+        cudaFree(g->biz_rank);
         g->biz_index = nullptr;
-        g->biz_hop2 = g->biz_radj = nullptr;
+        g->biz_hop2 = g->biz_radj = g->biz_rank = nullptr;
         return;
     }
     g->biz_index_words = words;
     g->biz_index_bytes = (int64_t)bytes;
-    g->device_bytes += (int64_t)bytes + (int64_t)sizeof(int) * (g->n_biz + g->u_adj_len);
+    g->device_bytes += (int64_t)bytes + (int64_t)sizeof(int) * (2 * (int64_t)g->n_biz + g->u_adj_len);
 }
 
-// Fills the reserved index: business ranks by degree (descending, ties by id), the ranked copy of
-// the user rows, then the rows.
+// Fills the reserved index: business ranks by degree (descending, ties by id, kept on the handle:
+// the kernel reads rank(b) per pair), the ranked copy of the user rows, then the rows.
 int build_biz_index(blp_graph* g, const int* b_deg_host) {
     if (!g->biz_index) return BLP_OK;
     const int n_biz = g->n_biz, words = g->biz_index_words;
@@ -215,18 +278,15 @@ int build_biz_index(blp_graph* g, const int* b_deg_host) {
     const size_t smem = (size_t)words * 4;
     const int rc = kernel_ctas_per_sm((const void*)k_build_biz_index, g->device, kIndexBuildThreads, smem, nullptr);
     if (rc != BLP_OK) return rc;
-    int* d_rank = nullptr;
-    BLP_CUDA_TRY(cudaMalloc((void**)&d_rank, sizeof(int) * (size_t)n_biz));
-    cudaError_t e = cudaMemcpy(d_rank, rank.data(), sizeof(int) * (size_t)n_biz, cudaMemcpyHostToDevice);
+    cudaError_t e = cudaMemcpy(g->biz_rank, rank.data(), sizeof(int) * (size_t)n_biz, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) {
-        k_rank_ids<<<g->sm_count * 8, 256>>>(g->u_adj, g->u_adj_len, d_rank, n_biz, g->biz_radj);
+        k_rank_ids<<<g->sm_count * 8, 256>>>(g->u_adj, g->u_adj_len, g->biz_rank, n_biz, g->biz_radj);
         k_build_biz_index<<<std::min(n_biz, g->sm_count * 8), kIndexBuildThreads, smem>>>(
             n_biz, words, (const unsigned long long*)g->b_row, g->b_adj,
-            (const unsigned long long*)g->u_row, g->biz_radj, d_rank, g->biz_index, g->biz_hop2);
+            (const unsigned long long*)g->u_row, g->biz_radj, g->biz_rank, g->biz_index, g->biz_hop2);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
-    cudaFree(d_rank);
     if (e != cudaSuccess) return blp::cuda_fail(e, "building the business index", __FILE__, __LINE__);
     g->biz_index_build_ms =
         std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -243,7 +303,7 @@ int score_biz_indexed(blp_graph* g, const SideArgs& a, const int32_t* pair_u, co
     BLP_CUDA_TRY(cudaEventRecord(g->ev[BLP_SIDE_BUSINESS][1], st));
     k_score_biz_indexed<<<grid, kIndexScoreThreads, 0, st>>>(a, pair_b, pair_u, n, g->n_users, g->b_deg,
                                                             g->u_deg, g->biz_radj, g->biz_index,
-                                                            g->biz_hop2, g->biz_index_words);
+                                                            g->biz_hop2, g->biz_rank, g->biz_index_words);
     BLP_CUDA_TRY(cudaGetLastError());
     if (cudaEventRecord(g->ev[BLP_SIDE_BUSINESS][2], st) == cudaSuccess) g->ev_recorded[BLP_SIDE_BUSINESS] = true;
     stats.path = BLP_PATH_BIZ_INDEX;
